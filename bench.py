@@ -3,6 +3,7 @@
 agent-env-steps/sec at 1/2/4/8 B200 vs the reference CPU path).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload pp_hard_ic3net] [--impl b200|reference]
+                    [--dump-outputs DIR]
 
 A "step" is one lock-step pass of the hot path over the whole env batch of a GPU:
 obs gather -> encoder -> comm/LSTM/heads/sampling -> env step (+ auto-reset), i.e.
@@ -224,7 +225,6 @@ class ClockSampler(object):
 # ------------------------------------------------------------------------------
 def gpu_arm(opts):
     import ctypes as C
-    import statistics
 
     import numpy as np
     import torch
@@ -283,6 +283,7 @@ def gpu_arm(opts):
 
         def __init__(self, trn):
             self.trn, self.graphs, self.replayed = trn, {}, 0
+            self.last_t = None                               # record index of the last enqueued iteration
 
         def _capture(self, n):
             torch.cuda.synchronize()
@@ -318,6 +319,7 @@ def gpu_arm(opts):
                 else:
                     self.trn._enqueue(n)
                 done += n
+                self.last_t = n - 1
 
         def launches(self):
             return _lib.launch_count() + self.replayed
@@ -347,32 +349,24 @@ def gpu_arm(opts):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item()), (w0, w1)
 
-    def measure(run, reduce_stats=True, min_seconds=0.5, max_repeats=400):
-        """Repeat the K-step region until >= min_seconds of device time have been measured (at least 3 times):
-        the driver's K = 20 is an 11 ms region, too short for one number to mean anything.  Every region time is
-        already the max over ranks, so all ranks leave the loop together."""
-        times, windows, total = [], [], 0.0
-        while (total < min_seconds * 1e3 or len(times) < 3) and len(times) < max_repeats:
-            ms, win = timed_region(run, K, reduce_stats)
-            times.append(ms)
-            windows.append(win)
-            total += ms
-        return times, (windows[0][0], windows[-1][1])
-
-    # ---- warm-up + timed regions (value: inputs resident in HBM, no host sync before the statistics copy) ----
+    # ---- warm-up + ONE timed region of exactly K = --steps lock-step iterations (inputs resident in HBM, no host sync
+    #      before the statistics copy).  A fixed step count makes the state the region leaves -- what --dump-outputs
+    #      writes -- the same from run to run.  Warmed inside the clock sampler so the GPU does not idle before it, and
+    #      the statistics reduction the region ends with is warmed too (first launch, first copy). ----
     run = Runner(tr)
-    run.warm(W)
-    launches0 = run.launches()
     with ClockSampler(local) as clk:
-        times, window = measure(run)
+        run.warm(W)
+        mgt.reduce_device(None, with_grads=True)
+        launches0 = run.launches()
+        ms, window = timed_region(run, K, True)
         time.sleep(0.2)
-    launches = (run.launches() - launches0) // max(1, len(times))
-    ms = statistics.median(times)
+    launches = run.launches() - launches0
     value = world * B * N * K / (ms * 1e-3)
-    timing = dict(repeats=len(times), ms_median=ms, ms_min=min(times), ms_max=max(times),
-                  region="K lock-step iterations + device stat reduction"
-                         + (" + all-reduce(flat_grads) + all-reduce(stat vector)" if world > 1 else "")
-                         + " + 1 D2H stat copy; value uses the median region")
+    timing = dict(ms=ms, region="K lock-step iterations + device stat reduction"
+                                + (" + all-reduce(flat_grads) + all-reduce(stat vector)" if world > 1 else "")
+                                + " + 1 D2H stat copy")
+    if opts.dump_outputs and rank == 0:
+        dump_outputs(opts.dump_outputs, tr, run.last_t)
 
     # ---- full training update: MultiGPUTrainer.train_batch on every rank (rollout with the reference batch boundary
     #      + compute_grad + gradient / statistics all-reduce + RMSprop), SURVEY 8(f)-1/2 + 8(e) ----
@@ -477,9 +471,8 @@ def gpu_arm(opts):
             a2, env2, net2, tr2 = build("index")
             run2 = Runner(tr2)
             run2.warm(W)
-            t2, _ = measure(run2, reduce_stats=False, min_seconds=0.25)
-            ms2 = statistics.median(t2)
-            alt = dict(obs_mode="index", value=B * N * K / (ms2 * 1e-3), ms_per_step=ms2 / K, repeats=len(t2),
+            ms2, _ = timed_region(run2, K, False)
+            alt = dict(obs_mode="index", value=B * N * K / (ms2 * 1e-3), ms_per_step=ms2 / K,
                        note="same rollout with the encoder evaluated from the env state (bit-identical x); "
                             "this is Trainer's default obs_mode")
             del tr2, net2, env2, run2
@@ -525,6 +518,28 @@ def gpu_arm(opts):
         dist.barrier()
         dist.destroy_process_group()
     return 0
+
+
+HIDDEN_SAMPLE_SLOTS = 1024       # env slots of the hidden state written by --dump-outputs (all of them: 84 MB at PP hard)
+
+
+def dump_outputs(path, tr, t):
+    """Write what the rollout handed its caller in its last lock-step iteration (record index t) as <path>/<name>.npy:
+    the RolloutBatch fields of that iteration and the merged statistics vector in full, the LSTM state (h, c) for a
+    fixed seeded sample of env slots.  float32 (integers and masks are exact in it), float64 for the statistics."""
+    import numpy as np
+    import torch
+    b, B, N = tr._buf, tr.env.env.nenvs, tr.args.nagents
+    out = dict(action=b["action"][t], logp=b["logp"][t], value=b["value"][t].view(B, N), reward=b["reward"][t],
+               episode_mask=b["emask"][t], episode_mini_mask=b["mini"][t], alive_mask=b["ralive"][t],
+               valid=b["valid"][t])
+    slots = np.sort(np.random.default_rng(0).choice(B, size=min(B, HIDDEN_SAMPLE_SLOTS), replace=False))
+    idx = torch.as_tensor(slots, device=b["h"].device)
+    out.update(h=b["h"].view(B, N, -1)[idx], c=b["c"].view(B, N, -1)[idx])
+    os.makedirs(path, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(path, k + ".npy"), v.float().cpu().numpy())
+    np.save(os.path.join(path, "stat.npy"), b["statvec"].cpu().numpy())
 
 
 def train_leg(opts, build, MultiGPUTrainer, world, dev, dist, torch):
@@ -806,7 +821,12 @@ def main():
     ap.add_argument("--obs_chunk_mb", type=float, default=0.0,
                     help="dense rollout: gather + encode observations in chunks of env slots of at most this size "
                          "(experiment; 0 = the whole batch at once, the measured optimum)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last of them computed (rank 0's env slots) as "
+                         "DIR/<name>.npy; the same arguments give the same inputs on every run")
     opts = ap.parse_args()
+    if opts.dump_outputs and opts.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b200 implementation")
     if opts.impl == "reference":
         return reference_arm(opts)
     return gpu_arm(opts)

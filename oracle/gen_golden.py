@@ -468,6 +468,13 @@ def gen_episode_case(name, seed, env_ids, wseed, hsteps=(0, 1), epoch=0, **kw):
 # 5. REINFORCE gradient of a whole batch through the reference's Trainer.run_batch + compute_grad
 # --------------------------------------------------------------------------
 def gen_grad_case(name, seed, env_id, wseed, **kw):
+    meta, arrays = ref_grad_case(seed, env_id, wseed, **kw)
+    save(name, meta, **arrays)
+
+
+def ref_grad_case(seed, env_id, wseed, full_grads=False, **kw):
+    """(meta, arrays) of one reference worker's run_batch + compute_grad, checked against oracle/grad.py.  Gradients
+    larger than 4096 values are stored as a sample + sums unless ``full_grads``."""
     import torch
     from . import grad as ograd
     from .rollout import run_episode
@@ -527,7 +534,7 @@ def gen_grad_case(name, seed, env_id, wseed, **kw):
             continue
         scale = max(1.0, float(np.abs(rg).max()))
         assert np.allclose(g[key], rg, rtol=1e-8, atol=1e-9 * scale), (name, key, np.abs(g[key] - rg).max())
-        if rg.size <= 4096:
+        if rg.size <= 4096 or full_grads:
             arrays["g_" + key] = rg
         else:
             arrays["gsum_" + key] = np.array([rg.sum(), np.abs(rg).sum(), (rg ** 2).sum()])
@@ -541,7 +548,7 @@ def gen_grad_case(name, seed, env_id, wseed, **kw):
     if is_tj:
         arrays["grid"] = tables["grid"]
         arrays["route_len"], arrays["route_cells"] = pack_routes(tables["routes"])
-    save(name, meta, **arrays)
+    return meta, arrays
 
 
 def gen_rmsprop_case(name, seed, nupdates=5, lr=0.001):
@@ -610,6 +617,72 @@ def gen_log_case(name="log_contract"):
     out = dict(epochs=epochs, lines=lines, log={k: [conv(x) for x in f.data] for k, f in log.items()})
     with open(os.path.join(GOLDEN, name + ".json"), "w") as f:
         json.dump(out, f, indent=0)
+
+
+def _load_path(modname, path):
+    import importlib.util
+    spec = importlib.util.spec_from_file_location(modname, path)
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
+
+
+def _test_cases(name):
+    """A module of tests/, loaded by path: the cases a fixture is recorded for are defined once, in the test."""
+    return _load_path("_cases_" + name, os.path.join(os.path.dirname(GOLDEN), name + ".py"))
+
+
+def _write_json(name, out):
+    path = os.path.join(GOLDEN, name + ".json")
+    with open(path, "w") as f:
+        json.dump(out, f, indent=0)
+    print("wrote %-40s %7.1f KB" % (name + ".json", os.path.getsize(path) / 1024.0))
+
+
+def gen_host_logic_case(name="host_logic"):
+    """What the reference's merge_stat (utils.py:15-29), parse_action_args (action_utils.py:5-25) and GymWrapper
+    properties (env_wrappers.py:21-50) return for the cases of tests/test_host_logic.py -> tests/golden/host_logic.json."""
+    import copy
+    t = _test_cases("test_host_logic")
+    ref_shims.install()
+    import gym.spaces as gspaces                      # the stub installed by ref_shims
+    ref = {m: _load_path("_ref_" + m, os.path.join(ref_shims.REF_ROOT, m + ".py"))
+           for m in ("utils", "action_utils", "env_wrappers")}
+    merged = []
+    for src, dest in t.STAT_CASES:
+        d = copy.deepcopy(dest)
+        ref["utils"].merge_stat(copy.deepcopy(src), d)
+        merged.append({k: t.typed(v) for k, v in d.items()})
+    actions = [t._run(ref["action_utils"].parse_action_args, kw) for kw in t.ACTION_CASES]
+    wrapper = {}
+    for kind in ("pp", "tj", "multi"):
+        w = ref["env_wrappers"].GymWrapper(t._FakeEnv(gspaces, kind))
+        wrapper[kind] = [int(w.observation_dim), int(w.num_actions), int(w.dim_actions)]
+    _write_json(name, dict(merge_stat=merged, parse_action_args=actions, gym_wrapper=wrapper))
+
+
+def gen_log_main_py_case(name="log_main_py"):
+    """The reference's log table (main.py:190-201: keys, plot flags, x axes, divisors) and what its main.py statements
+    (oracle/ref_log.py) log and print for the epochs of tests/test_log_contract.py -> tests/golden/log_main_py.json."""
+    import copy
+    from . import ref_log
+    t = _test_cases("test_log_contract")
+    log = ref_log.make_log()
+    lines = [ref_log.epoch_update(log, copy.deepcopy(st), 1.2345) for st in t.main_py_epochs()]
+    _write_json(name, dict(keys=list(log.keys()), fields={k: [f.plot, f.x_axis, f.divide_by] for k, f in log.items()},
+                           log={k: [t.to_jsonable(x) for x in f.data] for k, f in log.items()}, lines=lines))
+
+
+def gen_apa_case(name="apa_pp_ic3net"):
+    """--advantages_per_action off and on (trainer.py:189-199): the reference's losses and gradients for both settings
+    on the same episodes, each checked against oracle/grad.py (which has no such flag) before it is written."""
+    kw = dict(env_name="predator_prey", nagents=3, dim=5, vision=1, max_steps=8, hid_size=16, ic3net=True,
+              batch_size=16)
+    meta, arrays = ref_grad_case(19, 0, 7, full_grads=True, advantages_per_action=False, **kw)
+    meta_on, on = ref_grad_case(19, 0, 7, full_grads=True, advantages_per_action=True, **kw)
+    meta["on"] = {k: meta_on[k] for k in ("action_loss", "value_loss", "entropy", "num_steps", "num_episodes")}
+    arrays.update({"on_" + k: v for k, v in on.items() if k.startswith("g_")})
+    save(name, meta, **arrays)
 
 
 def gen_variant_case(name, seed, obs_dim, heads, model, nrep=4, use_alive=False, **kw):
@@ -797,6 +870,13 @@ def main():
     if "--log-only" in sys.argv:
         gen_log_case()
         return 0
+    if "--host-only" in sys.argv:
+        import warnings
+        warnings.filterwarnings("ignore")
+        gen_host_logic_case()
+        gen_log_main_py_case()
+        gen_apa_case()
+        return 0
     if "--rmsprop-only" in sys.argv:          # needs torch only, not the reference checkout
         gen_rmsprop_case("rmsprop_ref", 81)
         return 0
@@ -867,6 +947,9 @@ def main():
     gen_variant_cases()
     gen_rmsprop_case("rmsprop_ref", 81)
     gen_log_case()
+    gen_host_logic_case()
+    gen_log_main_py_case()
+    gen_apa_case()
     return 0
 
 

@@ -1,9 +1,9 @@
 """CPU tests of the host-side glue the rollout's callers rely on: merge_stat (utils.py:15-29) and
-parse_action_args (action_utils.py:5-25) -- fixed expectations, plus a differential check against the reference's
-own functions when /root/reference is present (it is in the build container, not on the GPU box)."""
+parse_action_args (action_utils.py:5-25) -- fixed expectations, plus a differential check against what the reference's
+own functions return for the same cases (tests/golden/host_logic.json, recorded by oracle/gen_golden.py)."""
 import argparse
 import copy
-import importlib.util
+import json
 import os
 
 import numpy as np
@@ -12,17 +12,12 @@ import pytest
 from ic3net_b200.action_utils import parse_action_args
 from ic3net_b200.utils import merge_stat
 
-REF = "/root/reference"
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
-def _ref_module(name):
-    path = os.path.join(REF, name + ".py")
-    if not os.path.exists(path):
-        return None
-    spec = importlib.util.spec_from_file_location("_ref_" + name, path)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
+def _golden(name):
+    with open(os.path.join(GOLDEN, name + ".json")) as f:
+        return json.load(f)
 
 
 STAT_CASES = [
@@ -37,13 +32,15 @@ STAT_CASES = [
 ]
 
 
-def _same(a, b):
-    assert a.keys() == b.keys()
-    for k in a:
-        if isinstance(a[k], np.ndarray) or isinstance(b[k], np.ndarray):
-            assert np.array_equal(a[k], b[k]) and type(a[k]) is type(b[k]), k
-        else:
-            assert a[k] == b[k] and type(a[k]) is type(b[k]), k
+def typed(x):
+    """JSON form of a merged value that keeps its type apart (bool / int / float / str, ndarray dtype, nesting)."""
+    if isinstance(x, np.ndarray):
+        return ["ndarray", str(x.dtype), x.tolist()]
+    if isinstance(x, list):
+        return ["list", [typed(v) for v in x]]
+    if isinstance(x, np.generic):
+        return [type(x).__name__, x.item()]
+    return [type(x).__name__, x]
 
 
 def test_merge_stat_rules():
@@ -64,14 +61,11 @@ def test_merge_stat_rules():
 
 @pytest.mark.parametrize("case", range(len(STAT_CASES)))
 def test_merge_stat_matches_reference(case):
-    ref = _ref_module("utils")
-    if ref is None:
-        pytest.skip("reference checkout not present")
     src, dest = STAT_CASES[case]
-    d1, d2 = copy.deepcopy(dest), copy.deepcopy(dest)
-    merge_stat(copy.deepcopy(src), d1)
-    ref.merge_stat(copy.deepcopy(src), d2)
-    _same(d1, d2)
+    d = copy.deepcopy(dest)
+    merge_stat(copy.deepcopy(src), d)
+    ours = json.loads(json.dumps({k: typed(v) for k, v in d.items()}))
+    assert ours == _golden("host_logic")["merge_stat"][case]
 
 
 ACTION_CASES = [
@@ -108,10 +102,8 @@ def test_parse_action_args_rules():
 
 @pytest.mark.parametrize("case", range(len(ACTION_CASES)))
 def test_parse_action_args_matches_reference(case):
-    ref = _ref_module("action_utils")
-    if ref is None:
-        pytest.skip("reference checkout not present")
-    assert _run(parse_action_args, ACTION_CASES[case]) == _run(ref.parse_action_args, ACTION_CASES[case])
+    ours = json.loads(json.dumps(_run(parse_action_args, ACTION_CASES[case])))
+    assert ours == _golden("host_logic")["parse_action_args"][case]
 
 
 # ---- GymWrapper on duck-typed environments (no GPU needed) ---------------------------------------------
@@ -178,17 +170,12 @@ def test_gym_wrapper_surface(kind, odim, nact, dact):
 
 @pytest.mark.parametrize("kind", ["pp", "tj", "multi"])
 def test_gym_wrapper_matches_reference_properties(kind):
-    """observation_dim / num_actions / dim_actions against the reference's GymWrapper on the same space objects."""
-    from oracle import ref_shims
-    if not ref_shims.reference_available():
-        pytest.skip("reference checkout not present")
-    ref_shims.install()
-    import gym.spaces as gspaces                      # the stub installed by ref_shims
-    ref = _ref_module("env_wrappers")
+    """observation_dim / num_actions / dim_actions against the reference's GymWrapper on the same space objects (the
+    gym space stand-ins of oracle/ref_shims.py, which the reference ran on when the fixture was recorded)."""
     from ic3net_b200.env_wrappers import GymWrapper
-    env = _FakeEnv(gspaces, kind)
-    a, b = GymWrapper(env), ref.GymWrapper(env)
-    assert (a.observation_dim, a.num_actions, a.dim_actions) == (b.observation_dim, b.num_actions, b.dim_actions)
+    from oracle.ref_shims import _make_gym_stub
+    a = GymWrapper(_FakeEnv(_make_gym_stub()["gym.spaces"], kind))
+    assert [a.observation_dim, a.num_actions, a.dim_actions] == _golden("host_logic")["gym_wrapper"][kind]
 
 
 def test_enemy_comm_derived_args_and_stat_split():
@@ -223,51 +210,31 @@ def test_enemy_comm_derived_args_and_stat_split():
 def test_advantages_per_action_is_the_same_loss_in_the_reference():
     """--advantages_per_action (trainer.py:189-199) multiplies the advantage into every head's log-probability before the
     sum instead of after it: the loss -- and therefore the gradient -- is the same number.  This repo accepts the flag and
-    has one code path; the claim is pinned here on the unmodified reference (skipped where it is not present)."""
-    from oracle import ref_shims
-    if not ref_shims.reference_available():
-        pytest.skip("reference checkout not present")
-    import torch
-    from oracle.gen_golden import RefRandom, make_weights, routed
-    ref_shims.install()
-    prev = torch.get_default_dtype()
-    torch.set_default_dtype(torch.float64)
-    try:
-        from comm import CommNetMLP
-        from trainer import Trainer
-        out = []
-        for flag in (False, True):
-            a = ref_shims.make_args(env_name="predator_prey", nagents=3, dim=5, vision=1, max_steps=8, hid_size=16,
-                                    ic3net=True, batch_size=16, advantages_per_action=flag)
-            w = ref_shims.make_ref_env(a)
-            ref_shims.finish_args(a, w)
-            net = CommNetMLP(a, a.num_inputs)
-            sd = make_weights(7, a.num_inputs, a.hid_size, a.naction_heads, a.comm_init)
-            net.load_state_dict({k: torch.from_numpy(v) for k, v in sd.items()})
-            tr = Trainer(a, net, w)
-            rr = RefRandom(19, 0)
-            orig_step, orig_reset = w.step, w.reset
-
-            def step(action, _o=orig_step, _rr=rr):
-                _rr.group = -1
-                o = _o(action)
-                _rr.tick += 1
-                _rr.head = 0
-                return o
-
-            def reset(epoch, _o=orig_reset, _rr=rr):
-                o = _o(epoch)
-                _rr.episode += 1
-                return o
-            w.step, w.reset = step, reset
-            with routed(rr):
-                batch, stat = tr.run_batch(0)
-            tr.optimizer.zero_grad()
-            s = tr.compute_grad(batch)
-            out.append((s, {k: v.grad.clone() for k, v in net.named_parameters() if v.grad is not None}))
-        (s0, g0), (s1, g1) = out
-        assert np.isclose(s0["action_loss"], s1["action_loss"], rtol=1e-12, atol=1e-12)
-        for k in g0:
-            assert torch.allclose(g0[k], g1[k], rtol=1e-10, atol=1e-12), k
-    finally:
-        torch.set_default_dtype(prev)
+    has one code path.  The fixture holds the unmodified reference's losses and gradients with the flag off and on, on
+    the same episodes: they agree, and the float64 oracle (oracle/grad.py) reproduces both."""
+    from helpers import load_golden, make_oracle_env, ns
+    from oracle import grad as ograd
+    from oracle import policy
+    from oracle.gen_golden import make_weights
+    from oracle.rollout import run_episode
+    meta, z = load_golden("apa_pp_ic3net")
+    assert not meta["args"]["advantages_per_action"]
+    for k in ("action_loss", "value_loss", "entropy"):
+        assert np.isclose(meta[k], meta["on"][k], rtol=1e-12, atol=1e-12), k
+    args = ns(meta["args"])
+    p = policy.params_to_f64(make_weights(meta["weights_seed"], meta["obs_dim"], args.hid_size, meta["heads"],
+                                          args.comm_init))
+    env = make_oracle_env(args)
+    eps, tick = [], 0
+    while tick < meta["num_steps"]:
+        eps.append(run_episode(env, p, args, meta["seed"], meta["env_id"], epoch=0, tick0=tick, episode=len(eps)))
+        tick += eps[-1]["num_steps"]
+    assert len(eps) == meta["num_episodes"] == meta["on"]["num_episodes"]
+    g, st, _ = ograd.compute_grad(p, eps, args)
+    for k in ("action_loss", "value_loss", "entropy"):
+        assert np.isclose(st[k], meta[k], rtol=1e-9, atol=1e-9), k
+    keys = [k for k in z.files if k.startswith("g_")]
+    assert len(keys) >= 8 and sorted("on_" + k for k in keys) == sorted(k for k in z.files if k.startswith("on_"))
+    for key in keys:
+        assert np.allclose(z[key], z["on_" + key], rtol=1e-10, atol=1e-12), key
+        assert np.allclose(g[key[2:]], z[key], rtol=1e-8, atol=1e-10), key

@@ -1,8 +1,8 @@
 """SURVEY 8(f)-3: the stat / log pipeline the hot path's callers rely on.
 
-(1) differential: ic3net_b200.main.update_log / epoch_lines against the reference's own main.py statements
-    (oracle/ref_log.py executes main.py:190-201,218-244 from the unmodified source text) on randomised epoch stats,
-    including fields an epoch did not produce and zero divisors;
+(1) differential: ic3net_b200.main.update_log / epoch_lines against what the reference's own main.py statements
+    (oracle/ref_log.py executes main.py:190-201,218-244 from the unmodified source text) logged and printed for
+    randomised epoch stats, including fields an epoch did not produce and zero divisors (tests/golden/log_main_py.json);
 (2) the same against a committed fixture of reference outputs (tests/golden/log_contract.json), so the contract is
     checked where the reference is absent;
 (3) 1-rank vs 2-rank: statistics merged over ranks with the reference's merge rule give the same per-epoch values
@@ -14,13 +14,12 @@ import os
 import sys
 
 import numpy as np
-import pytest
 
 from ic3net_b200 import main as m
 from ic3net_b200.utils import LogField, merge_stat
-from oracle import ref_shims
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "log_contract.json")
+GOLDEN_MAIN_PY = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "log_main_py.json")
 
 
 def random_epoch(rs, nagents, kind):
@@ -55,22 +54,21 @@ def run_ours(epochs):
     return {k: [to_jsonable(x) for x in v.data] for k, v in log.items()}, lines
 
 
-@pytest.mark.skipif(not ref_shims.reference_available(), reason="reference sources not present")
-def test_update_log_matches_reference_main_py_text():
-    from oracle import ref_log
+def main_py_epochs():
     rs = np.random.RandomState(3)
-    epochs = [random_epoch(rs, 4, kind) for kind in ("pp", "tj", "plain", "empty", "tj", "pp")]
-    ours, our_lines = run_ours(epochs)
-    log = ref_log.make_log()
-    ref_lines = []
-    for st in epochs:
-        ref_lines.append(ref_log.epoch_update(log, copy.deepcopy(st), 1.2345))
-    assert list(log.keys()) == list(m.make_log().keys())
-    for k, f in log.items():
-        mine = m.make_log()[k]
-        assert (f.plot, f.x_axis, f.divide_by) == (mine.plot, mine.x_axis, mine.divide_by), k
-        assert json.dumps([to_jsonable(x) for x in f.data]) == json.dumps(ours[k]), k
-    assert ref_lines == our_lines
+    return [random_epoch(rs, 4, kind) for kind in ("pp", "tj", "plain", "empty", "tj", "pp")]
+
+
+def test_update_log_matches_reference_main_py_text():
+    with open(GOLDEN_MAIN_PY) as f:
+        fx = json.load(f)
+    ours, our_lines = run_ours(main_py_epochs())
+    mine = m.make_log()
+    assert list(mine.keys()) == fx["keys"]
+    for k, f in mine.items():
+        assert [f.plot, f.x_axis, f.divide_by] == fx["fields"][k], k
+        assert json.dumps(fx["log"][k]) == json.dumps(ours[k]), k
+    assert fx["lines"] == our_lines
 
 
 def test_update_log_matches_committed_reference_fixture():
