@@ -17,7 +17,7 @@ MAX_HEADS = 4
 MAX_HEAD_DIM = 16
 MAX_PASSES = 4
 CELL_LSTM, CELL_TANH = 0, 1
-LSTM_IMG_BYTES = 1572864
+LSTM_IMG_BYTES = 786432
 
 ERR_EPISODE_DONE = 1
 ERR_ROUTE_OVERRUN = 2
@@ -49,8 +49,7 @@ class RolloutIO(C.Structure):
                 ("reserved0", C.c_int32), ("halted", _p), ("rec_valid", _p), ("snap_T", C.c_int32),
                 ("reserved1", C.c_int32), ("snap_fresh", _p), ("snap_comm", _p), ("snap_alive", _p), ("snap_tep", _p),
                 ("snap_pp_loc", _p), ("snap_tj_loc", _p), ("snap_tj_alive", _p), ("snap_tj_last_act", _p),
-                ("snap_tj_route_id", _p), ("head_partial", _p), ("head_b", _p), ("head_value", _p), ("head_logp", _p),
-                ("head_dim", C.c_int32 * MAX_HEADS)]
+                ("snap_tj_route_id", _p)]
 
 
 class TJCfg(C.Structure):
@@ -89,7 +88,7 @@ class PolicyIO(C.Structure):
     _fields_ = [("x", _p), ("h", _p), ("c", _p), ("comm_action", _p), ("alive", _p), ("fresh", _p), ("tick", _p),
                 ("draws", _p), ("h_out", _p), ("c_out", _p), ("value", _p), ("logp", _p), ("action", _p),
                 ("workspace", _p), ("err", _p), ("pp_env", _p), ("pp_state", _p), ("tj_env", _p), ("tj_state", _p),
-                ("x_table", _p), ("defer_heads", C.c_int32), ("pass_index", C.c_int32)]
+                ("x_table", _p), ("pass_index", C.c_int32)]
 
 
 class BpttPlan(C.Structure):
@@ -129,7 +128,6 @@ SYMBOLS = {
     "ic3_tj_encoder_table": (C.c_int, [C.POINTER(TJCfg), C.POINTER(PolicyCfg), C.POINTER(PolicyPacked), _PTR, _PTR]),
     "ic3_policy_workspace_bytes": (C.c_uint64, [C.POINTER(PolicyCfg)]),
     "ic3_policy_step": (C.c_int, [C.POINTER(PolicyCfg), C.POINTER(PolicyPacked), C.POINTER(PolicyIO), _PTR]),
-    "ic3_policy_partial_ptr": (C.c_void_p, [C.POINTER(PolicyCfg), _PTR]),
     "ic3_policy_step_profile": (C.c_int, [C.POINTER(PolicyCfg), C.POINTER(PolicyPacked), C.POINTER(PolicyIO), _PTR,
                                           C.POINTER(C.c_float)]),
     "ic3_sample_actions": (C.c_int, [C.POINTER(PolicyCfg), _PTR, _PTR, _PTR, _PTR, _PTR]),

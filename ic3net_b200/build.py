@@ -36,7 +36,7 @@ def _stale():
 def build(force=False, verbose=False):
     if not force and not _stale():
         return LIB
-    extra = os.environ.get("IC3_NVCC_EXTRA", "").split()      # profiling experiments only (e.g. -DIC3_TC_EXP_SKIP_MMA)
+    extra = os.environ.get("IC3_NVCC_EXTRA", "").split()      # extra nvcc flags for local experiments
     objs = []
     procs = []
     for src in SOURCES:

@@ -1307,7 +1307,8 @@ static int bptt_prepare_on(const ic3_bptt_plan* p, const ic3_bptt_step_io* io, c
     src.pp = *p->pp_env;
     memset(&src.pps, 0, sizeof(src.pps));
     src.pps.loc = const_cast<int32_t*>(io->pp_loc);
-    IC3_LAUNCH_RC(ic3_launch_pdl(prep_kernel<XSRC_PP, true, true>, dim3(2 * ntiles), dim3(PREP_THREADS), prep_T_bytes(cfg->N), s, *cfg, pio, a_img, src, bw));
+    prep_kernel<XSRC_PP, true, true><<<2 * ntiles, PREP_THREADS, prep_T_bytes(cfg->N), s>>>(*cfg, pio, a_img, src, bw);
+    IC3_LAUNCH_CHECK();
     trace_mark(1, io->t, s);
   } else {
     if (!io->tj_loc || !io->tj_alive || !io->tj_last_act || !io->tj_route_id) return IC3_E_NULL;
@@ -1317,7 +1318,8 @@ static int bptt_prepare_on(const ic3_bptt_plan* p, const ic3_bptt_step_io* io, c
     src.tjs.alive = const_cast<uint8_t*>(io->tj_alive);
     src.tjs.last_act = const_cast<uint8_t*>(io->tj_last_act);
     src.tjs.route_id = const_cast<int32_t*>(io->tj_route_id);
-    IC3_LAUNCH_RC(ic3_launch_pdl(prep_kernel<XSRC_TJ, true, true>, dim3(2 * ntiles), dim3(PREP_THREADS), prep_T_bytes(cfg->N), s, *cfg, pio, a_img, src, bw));
+    prep_kernel<XSRC_TJ, true, true><<<2 * ntiles, PREP_THREADS, prep_T_bytes(cfg->N), s>>>(*cfg, pio, a_img, src, bw);
+    IC3_LAUNCH_CHECK();
   }
   // ---- heads ----
   HeadsArgs ha;

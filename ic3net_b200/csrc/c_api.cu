@@ -1,21 +1,7 @@
 // Library-level entry points of the C ABI (include/ic3net_b200.h).
 #include "ic3_common.cuh"
 
-#include <cstdlib>
-
 unsigned long long g_ic3_launches = 0;
-
-// Programmatic dependent launch of the rollout kernels (ic3_common.cuh).  Measured on B200 (bench.py --quick, PP hard,
-// 8192 envs): index-form step 0.166 ms without vs 0.197 ms with, dense step 0.546 vs 0.635 ms -- the early-resident
-// dependent grids cost more than the ~1 us launch gaps they hide, so it is OFF unless IC3_PDL=1.
-bool ic3_pdl_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("IC3_PDL");
-    v = (e && atoi(e) != 0) ? 1 : 0;
-  }
-  return v == 1;
-}
 
 extern "C" const char* ic3_version(void) { return "ic3net_b200 0.1 (sm_100a)"; }
 

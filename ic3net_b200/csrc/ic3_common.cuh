@@ -20,44 +20,6 @@ extern unsigned long long g_ic3_launches;  // c_api.cu
     if (_e != cudaSuccess) return (int)_e;         \
   } while (0)
 
-// launch through a runtime call that returns the error (cudaLaunchKernelEx)
-#define IC3_LAUNCH_RC(expr)                                   \
-  do {                                                        \
-    ++g_ic3_launches;                                         \
-    cudaError_t _e = (expr);                                  \
-    if (_e == cudaSuccess) _e = cudaGetLastError();           \
-    if (_e != cudaSuccess) return (int)_e;                    \
-  } while (0)
-
-// ---------------------------------------------------------------------------
-// Programmatic dependent launch (sm_90+): the kernels of a rollout step form a dependent chain
-// (prep -> lstm -> heads -> env step -> next prep ...).  Launched with the programmatic-serialization
-// attribute, the next grid's CTAs are scheduled as soon as every CTA of the current grid has passed
-// ic3_pdl_trigger() and SM resources are free; they block in ic3_pdl_wait() until the previous grid has
-// COMPLETED and its writes are visible.  Rule kept by every kernel: nothing that another kernel of the stream
-// writes (or that this kernel writes) is touched before ic3_pdl_wait().  Without the attribute (the default, see
-// ic3_pdl_enabled() in c_api.cu for the measurement; or plain <<<>>> launches) both instructions are no-ops.
-// ---------------------------------------------------------------------------
-__device__ __forceinline__ void ic3_pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void ic3_pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
-bool ic3_pdl_enabled();   // c_api.cu: environment variable IC3_PDL (default 0)
-
-template <typename... KArgs, typename... Args>
-inline cudaError_t ic3_launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args... args) {
-  cudaLaunchConfig_t lc{};
-  lc.gridDim = grid;
-  lc.blockDim = block;
-  lc.dynamicSmemBytes = smem;
-  lc.stream = s;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  lc.attrs = at;
-  lc.numAttrs = ic3_pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&lc, kern, static_cast<KArgs>(args)...);
-}
-
 // ---------------------------------------------------------------------------
 // Philox4x32-10 (Salmon et al., SC'11).  Same stream layout as oracle/philox.py:
 //   key = (seed_lo, seed_hi), counter = (env_id, tick, stream, index)

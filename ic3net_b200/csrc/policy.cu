@@ -383,8 +383,6 @@ __global__ void __launch_bounds__(256) encoder_dense_kernel(const float* __restr
   constexpr int CPT = H / 32;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int row = blockIdx.x * (blockDim.x >> 5) + warp;
-  ic3_pdl_trigger();
-  ic3_pdl_wait();      // obs comes from the gather kernel launched just before
   if (row >= rows) return;
   float acc[CPT], acc2[CPT];
 #pragma unroll
@@ -694,12 +692,9 @@ int launch_encoder_dense(const ic3_policy_cfg* cfg, const ic3_policy_packed* w, 
   const bool vec = (cfg->O % 4 == 0) && ((reinterpret_cast<uintptr_t>(obs) & 15) == 0);
   const int grid = (rows + 7) / 8;
   const ObsLayout lay{cfg->obs_off, cfg->obs_vocab, cfg->obs_ncount};
-  if (vec)
-    IC3_LAUNCH_RC(ic3_launch_pdl(encoder_dense_kernel<H, true>, dim3(grid), dim3(256), 0, s, obs, (const float*)w->enc_wT,
-                                 (const float*)w->enc_b, x, rows, cfg->O, lay));
-  else
-    IC3_LAUNCH_RC(ic3_launch_pdl(encoder_dense_kernel<H, false>, dim3(grid), dim3(256), 0, s, obs, (const float*)w->enc_wT,
-                                 (const float*)w->enc_b, x, rows, cfg->O, lay));
+  if (vec) encoder_dense_kernel<H, true><<<grid, 256, 0, s>>>(obs, w->enc_wT, w->enc_b, x, rows, cfg->O, lay);
+  else encoder_dense_kernel<H, false><<<grid, 256, 0, s>>>(obs, w->enc_wT, w->enc_b, x, rows, cfg->O, lay);
+  IC3_LAUNCH_CHECK();
   return IC3_OK;
 }
 

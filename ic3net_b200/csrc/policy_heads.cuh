@@ -1,6 +1,6 @@
 // Value / action heads, log-softmax and inverse-CDF sampling for one agent row, executed by
-// one warp (reference: comm.py:228-239, action_utils.py:32-36).  Shared by the fp32 SIMT
-// policy kernel (policy.cu) and the tcgen05 policy path (policy_tc.cu).
+// one warp (reference: comm.py:228-239, action_utils.py:32-36), for the fp32 SIMT policy
+// kernel (policy.cu).
 #pragma once
 #include "ic3_common.cuh"
 
@@ -62,88 +62,6 @@ __device__ __forceinline__ void heads_for_row(const ic3_policy_cfg& cfg, const f
     head_logp_sample(mylogit, off, na, (float)u24 * 5.9604644775390625e-08f, do_sample, mylogp, act);
     if (lane >= off && lane < off + na) logp[grow * atot + (off - 1) + (lane - off)] = mylogp;
     if (do_sample && lane == 0) action[grow * cfg.nheads + k] = act;
-    off += na;
-  }
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// Finishing the heads from the per-slot partial logits of the tcgen05 LSTM epilogue (fixed summation order ->
-// deterministic): value, log-softmax per head, inverse-CDF sampling of ONE agent row by ONE thread.  Used by
-// heads_finish_kernel (policy_tc) and, fused, by the env step kernels (ic3_rollout_io.head_partial).
-// ---------------------------------------------------------------------------------------------------------------
-constexpr int IC3_HEAD_PAD = 8;    // outputs (value + action logits) the fused epilogue supports
-constexpr int IC3_HEAD_NSLOT = 8;  // partial-logit slots per row
-
-struct HeadsFinish {
-  const float* partial;   // [R][IC3_HEAD_NSLOT][IC3_HEAD_PAD]
-  const float* head_b;    // [1 + sum(na)]
-  int nheads;
-  int head_dim[IC3_MAX_HEADS];
-  uint64_t seed;
-  uint32_t env_id0;
-  const uint32_t* tick;   // [B] or NULL
-  const uint32_t* draws;  // [R, nheads] or NULL
-  float* value;           // [R]
-  float* logp;            // [R, sum(na)]
-  int32_t* action;        // [R, nheads] or NULL (no sampling)
-};
-
-// returns the sampled action of the LAST head in *last_act / of head 0 in *first_act (env kernels consume head 0)
-__device__ __forceinline__ void heads_finish_row(const HeadsFinish& f, long row, int e, int i, int* first_act) {
-  float logit[IC3_HEAD_PAD];
-  const float4* p4 = reinterpret_cast<const float4*>(f.partial + (size_t)row * IC3_HEAD_NSLOT * IC3_HEAD_PAD);
-  {
-    float4 a = p4[0], b = p4[1];
-#pragma unroll
-    for (int sl = 1; sl < IC3_HEAD_NSLOT; ++sl) {
-      const float4 c = p4[2 * sl], d = p4[2 * sl + 1];
-      a.x += c.x; a.y += c.y; a.z += c.z; a.w += c.w;
-      b.x += d.x; b.y += d.y; b.z += d.z; b.w += d.w;
-    }
-    logit[0] = a.x; logit[1] = a.y; logit[2] = a.z; logit[3] = a.w;
-    logit[4] = b.x; logit[5] = b.y; logit[6] = b.z; logit[7] = b.w;
-  }
-  int atot = 0;
-  for (int k = 0; k < f.nheads; ++k) atot += f.head_dim[k];
-#pragma unroll
-  for (int o = 0; o < IC3_HEAD_PAD; ++o) logit[o] += (o < 1 + atot) ? __ldg(f.head_b + o) : 0.f;
-  f.value[row] = logit[0];
-  const bool do_sample = f.action != nullptr;
-  uint4 d24 = make_uint4(0, 0, 0, 0);
-  if (do_sample && !f.draws)
-    d24 = ic3_draw24(f.seed, f.env_id0 + (uint32_t)e, f.tick ? f.tick[e] : 0u, IC3_STREAM_ACTION, (uint32_t)i);
-  int off = 1;
-  for (int k = 0; k < f.nheads; ++k) {
-    const int na = f.head_dim[k];
-    float m = -INFINITY;
-#pragma unroll
-    for (int o = 1; o < IC3_HEAD_PAD; ++o)
-      if (o >= off && o < off + na) m = fmaxf(m, logit[o]);
-    float ssum = 0.f;
-#pragma unroll
-    for (int o = 1; o < IC3_HEAD_PAD; ++o)
-      if (o >= off && o < off + na) ssum += expf(logit[o] - m);
-    const float lse = m + logf(ssum);
-    uint32_t u24 = 0;
-    if (do_sample) u24 = f.draws ? f.draws[(size_t)row * f.nheads + k] : ic3_word(d24, k);
-    const float u = (float)u24 * 5.9604644775390625e-08f;
-    float cdf = 0.f;
-    int act = na - 1;
-    bool found = false;
-#pragma unroll
-    for (int o = 1; o < IC3_HEAD_PAD; ++o) {
-      if (o >= off && o < off + na) {
-        const float lp = logit[o] - lse;
-        f.logp[(size_t)row * atot + (o - 1)] = lp;
-        cdf += expf(lp);
-        if (!found && cdf > u) {
-          act = o - off;
-          found = true;
-        }
-      }
-    }
-    if (do_sample) f.action[(size_t)row * f.nheads + k] = act;
-    if (k == 0 && first_act) *first_act = act;
     off += na;
   }
 }

@@ -16,145 +16,48 @@
 // complete on an mbarrier, and the MMA descriptors are fixed offsets into the stage:
 //   prep kernel   x, h (fp32), gate masks  ->  A image [tile][12 chunks][hi,lo][4 kcore][16 rcore][8][8]
 //   pack kernel   weights                  ->  B image [2 halves][12 chunks][hi,lo][4 kcore][32 ncore][8][8]
-//   lstm kernel   one CTA per (128-row tile, 256-column half): warp 4 = bulk-copy producer +
-//                 TMEM allocator, warp 5 = MMA issuer (one thread), warps 0-3 = epilogue
-//                 (tcgen05.ld 32 lanes x 16 columns -> LSTM cell -> c', h'); 2 CTAs per SM
-//                 (256 TMEM columns, 97 KB smem each) overlap each other's prologue/epilogue.
-//   heads kernel  value / action heads + sampling from h' (warp per row).
+//   lstm kernel   persistent, one CTA per SM looping over work items (128-row tile, 256-column half):
+//                 warp 16 = bulk-copy producer (4-stage ring) + TMEM allocator, warp 17 = MMA issuer
+//                 (one thread) into two 256-column TMEM accumulators, warps 0-15 = epilogue
+//                 (tcgen05.ld -> LSTM cell -> c', h' + partial head logits) of item i while the
+//                 MMAs of item i+1 run.
+//   heads kernel  value / action heads + sampling: heads_finish_kernel sums the epilogue's partial
+//                 logits (thread per row, <= 7 action logits); heads_kernel<P> otherwise.
 #include "policy_tc_kernels.cuh"
 
 
-// Cluster size of the tensor-core kernel (CTAs sharing one weight stream).  Measured on B200: 1, 2 and 4 run at
-// the same speed (L2 already merges identical requests of neighbouring SMs), so 1 is the default; IC3_TC_CLUSTER
-// overrides it for experiments.
-static int tc_cluster_size() {
-  static int v = 0;
-  if (v == 0) {
-    const char* e = getenv("IC3_TC_CLUSTER");
-    v = e ? atoi(e) : 1;
-    if (v != 1 && v != 2 && v != 4 && v != 8) v = 1;
-  }
-  return v;
-}
-constexpr int TC_TILE_PAD = 8;   // tiles are padded to whole clusters of up to 8
-
-// IC3_TC_PAIR=1 selects the cta_group::2 kernel (one 2-SM MMA stream per CTA pair); experimental, default off.
-static bool tc_pair_mode() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("IC3_TC_PAIR");
-    v = (e && atoi(e) != 0) ? 1 : 0;
-  }
-  return v == 1;
-}
-
-static int launch_lstm_pair(const ic3_policy_cfg* cfg, const ic3_policy_io* io, const ic3_policy_packed* w,
-                            const __half* a_img, int ntiles_pad, int nout, float* partial, cudaStream_t s) {
-  static int max_clusters = 0;
-  const size_t smem = PAIR_NSTAGE * PAIR_STAGE_BYTES + 256 + TC_H * HEAD_PAD * sizeof(float) + 4 * TC_H * sizeof(float);
-  auto kern = lstm_tc_pair_kernel;
-  cudaLaunchAttribute la[2];
-  la[0].id = cudaLaunchAttributeClusterDimension;
-  la[0].val.clusterDim.x = 2; la[0].val.clusterDim.y = 1; la[0].val.clusterDim.z = 1;
-  if (max_clusters == 0) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return (int)e;
-    cudaLaunchConfig_t q{};
-    q.gridDim = dim3(2 * 148);
-    q.blockDim = dim3(TC_P_THREADS);
-    q.dynamicSmemBytes = smem;
-    q.attrs = la; q.numAttrs = 1;
-    e = cudaOccupancyMaxActiveClusters(&max_clusters, kern, &q);
-    if (e != cudaSuccess || max_clusters <= 0) return e != cudaSuccess ? (int)e : IC3_E_RANGE;
-  }
-  const int nitems = 2 * (ntiles_pad / 2);                         // (tile pair, column half)
-  const int nclusters = nitems < max_clusters ? nitems : max_clusters;
-  cudaLaunchConfig_t lc{};
-  lc.gridDim = dim3(nclusters * 2);
-  lc.blockDim = dim3(TC_P_THREADS);
-  lc.dynamicSmemBytes = smem;
-  lc.stream = s;
-  la[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  la[1].val.programmaticStreamSerializationAllowed = 1;
-  lc.attrs = la; lc.numAttrs = ic3_pdl_enabled() ? 2 : 1;
-  const __half* b_img = reinterpret_cast<const __half*>(w->lstm_img) + (size_t)io->pass_index * 2 * B_IMG_HALFS +
-                        B_IMG_HALFS;                                                  // the pair-layout copy
-  cudaError_t e = cudaLaunchKernelEx(&lc, kern, *cfg, *io, a_img, b_img,
-                                     (const float*)w->bias_cat + (size_t)io->pass_index * 4 * TC_H, nitems,
-                                     (const float*)w->head_w, nout, partial);
-  ++g_ic3_launches;
-  return e == cudaSuccess ? IC3_OK : (int)e;
-}
-
-template <int CL>
+// Persistent grid: as many CTAs as can be co-resident (one per SM: 148 on B200), each looping over work items.
 static int launch_lstm(const ic3_policy_cfg* cfg, const ic3_policy_io* io, const ic3_policy_packed* w, const __half* a_img,
-                       int ntiles_pad, size_t smem, int nout, float* partial, cudaStream_t s) {
-  static int max_clusters = 0;
-  auto kern = lstm_tc_kernel<CL>;
-  cudaLaunchAttribute la[2];
-  la[0].id = cudaLaunchAttributeClusterDimension;
-  la[0].val.clusterDim.x = CL; la[0].val.clusterDim.y = 1; la[0].val.clusterDim.z = 1;
-  if (max_clusters == 0) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+                       int ntiles, size_t smem, int nout, float* partial, cudaStream_t s) {
+  static int max_ctas = 0;
+  if (max_ctas == 0) {
+    cudaError_t e = cudaFuncSetAttribute(lstm_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
-    cudaLaunchConfig_t q{};
-    q.gridDim = dim3(CL * 148);
-    q.blockDim = dim3(TC_P_THREADS);
-    q.dynamicSmemBytes = smem;
-    q.attrs = la; q.numAttrs = 1;
-    e = cudaOccupancyMaxActiveClusters(&max_clusters, kern, &q);   // clusters that can be co-resident (persistent grid)
-    if (e != cudaSuccess || max_clusters <= 0) return e != cudaSuccess ? (int)e : IC3_E_RANGE;
+    int dev = 0, nsm = 0, per_sm = 0;
+    e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
+    if (e == cudaSuccess) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, lstm_tc_kernel, TC_P_THREADS, smem);
+    if (e != cudaSuccess) return (int)e;
+    if (per_sm <= 0) return IC3_E_RANGE;
+    max_ctas = nsm * per_sm;
   }
-  const int nitems = 2 * (ntiles_pad / CL);                        // (tile group, column half)
-  const int nclusters = nitems < max_clusters ? nitems : max_clusters;
-  cudaLaunchConfig_t lc{};
-  lc.gridDim = dim3(nclusters * CL);
-  lc.blockDim = dim3(TC_P_THREADS);
-  lc.dynamicSmemBytes = smem;
-  lc.stream = s;
-  la[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  la[1].val.programmaticStreamSerializationAllowed = 1;
-  lc.attrs = la; lc.numAttrs = ic3_pdl_enabled() ? 2 : 1;
-  const __half* b_img = reinterpret_cast<const __half*>(w->lstm_img) + (size_t)io->pass_index * 2 * B_IMG_HALFS;
-  cudaError_t e = cudaLaunchKernelEx(&lc, kern, *cfg, *io, a_img, b_img,
-                                     (const float*)w->bias_cat + (size_t)io->pass_index * 4 * TC_H, nitems,
-                                     (const float*)w->head_w, nout, partial);
-  ++g_ic3_launches;
-  return e == cudaSuccess ? IC3_OK : (int)e;
+  const int nitems = 2 * ntiles;                                   // (row tile, column half)
+  const int grid = nitems < max_ctas ? nitems : max_ctas;
+  const __half* b_img = reinterpret_cast<const __half*>(w->lstm_img) + (size_t)io->pass_index * B_IMG_HALFS;
+  lstm_tc_kernel<<<grid, TC_P_THREADS, smem, s>>>(*cfg, *io, a_img, b_img, w->bias_cat + (size_t)io->pass_index * 4 * TC_H,
+                                                  nitems, w->head_w, nout, partial);
+  IC3_LAUNCH_CHECK();
+  return IC3_OK;
 }
-
-#ifdef IC3_TC_EXP_TRACE
-extern "C" int ic3_debug_tc_trace(unsigned long long* host) {      // experiment builds only; not part of the C ABI
-  cudaDeviceSynchronize();
-  return (int)cudaMemcpyFromSymbol(host, g_tc_trace, sizeof(unsigned long long) * 4 * 512);
-}
-extern "C" int ic3_debug_tc_trace_clear() {
-  static unsigned long long z[4 * 512];
-  return (int)cudaMemcpyToSymbol(g_tc_trace, z, sizeof(z));
-}
-#endif
 
 uint64_t ic3_tc_workspace_bytes(const ic3_policy_cfg* cfg) {
   if (!cfg || cfg->H != TC_H) return 0;
   const long R = (long)cfg->B * cfg->N;
   const long ntiles = (R + TC_M - 1) / TC_M;
-  const long ntiles_pad = (ntiles + TC_TILE_PAD - 1) / TC_TILE_PAD * TC_TILE_PAD;   // whole clusters of tiles
   // operand image + per-slot partial logits [R][NSLOT][HEAD_PAD] (+ comm_passes > 1: two (h, c) pairs that carry the
   // state from one pass to the next)
   const uint64_t carry = cfg->passes > 1 ? (uint64_t)4 * R * TC_H * sizeof(float) : 0;
-  return (uint64_t)ntiles_pad * TC_NCHUNK * A_CHUNK_BYTES + (uint64_t)R * NSLOT * HEAD_PAD * sizeof(float) + carry;
-}
-
-extern "C" const float* ic3_policy_partial_ptr(const ic3_policy_cfg* cfg, const void* workspace) {
-  if (!cfg || !workspace || cfg->H != TC_H) return nullptr;
-  int nout = 1;
-  for (int k = 0; k < cfg->nheads; ++k) nout += cfg->head_dim[k];
-  if (nout > HEAD_PAD) return nullptr;
-  const long R = (long)cfg->B * cfg->N;
-  const long ntiles = (R + TC_M - 1) / TC_M;
-  const long ntiles_pad = (ntiles + TC_TILE_PAD - 1) / TC_TILE_PAD * TC_TILE_PAD;
-  return reinterpret_cast<const float*>(reinterpret_cast<const unsigned char*>(workspace) +
-                                        (size_t)ntiles_pad * TC_NCHUNK * A_CHUNK_BYTES);
+  return (uint64_t)ntiles * TC_NCHUNK * A_CHUNK_BYTES + (uint64_t)R * NSLOT * HEAD_PAD * sizeof(float) + carry;
 }
 
 int ic3_tc_pack(const ic3_policy_cfg* cfg, const ic3_policy_params* p, const ic3_policy_packed* out, cudaStream_t s) {
@@ -169,7 +72,7 @@ int ic3_tc_pack(const ic3_policy_cfg* cfg, const ic3_policy_params* p, const ic3
     ic3_policy_params q = *p;
     if (ps > 0 && p->c_w_pass[ps]) q.c_w = p->c_w_pass[ps];
     if (ps > 0 && p->c_b_pass[ps]) q.c_b = p->c_b_pass[ps];
-    pack_tc_kernel<<<(total + 255) / 256, 256, 0, s>>>(q, reinterpret_cast<__half*>(out->lstm_img) + (size_t)ps * 2 * B_IMG_HALFS,
+    pack_tc_kernel<<<(total + 255) / 256, 256, 0, s>>>(q, reinterpret_cast<__half*>(out->lstm_img) + (size_t)ps * B_IMG_HALFS,
                                                        out->bias_cat + (size_t)ps * 4 * TC_H, out->flags);
     IC3_LAUNCH_CHECK();
   }
@@ -243,7 +146,6 @@ int ic3_tc_policy_step(const ic3_policy_cfg* cfg, const ic3_policy_packed* w, co
 static int tc_pass(const ic3_policy_cfg* cfg, const ic3_policy_packed* w, const ic3_policy_io* io, cudaStream_t s, bool last) {
   const long R = (long)cfg->B * cfg->N;
   const int ntiles = (int)((R + TC_M - 1) / TC_M);
-  const int ntiles_pad = (ntiles + TC_TILE_PAD - 1) / TC_TILE_PAD * TC_TILE_PAD;   // padding tiles are written as zeros
   __half* img = reinterpret_cast<__half*>(io->workspace);
   PrepSrc src;
   memset(&src, 0, sizeof(src));
@@ -255,7 +157,7 @@ static int tc_pass(const ic3_policy_cfg* cfg, const ic3_policy_packed* w, const 
   if (src.table && !src.split) return IC3_E_RANGE;      // the table IS the first of the two sums
   prof_mark(0, s);
   if (io->x) {
-    IC3_LAUNCH_RC(ic3_launch_pdl(prep_kernel<XSRC_TENSOR, false>, dim3(2 * ntiles_pad), dim3(PREP_THREADS), prep_T_bytes(cfg->N), s, *cfg, *io, img, src, PrepBwd{}));
+    prep_kernel<XSRC_TENSOR, false><<<2 * ntiles, PREP_THREADS, prep_T_bytes(cfg->N), s>>>(*cfg, *io, img, src, PrepBwd{});
   } else if (io->pp_env && io->pp_state) {       // fused index encoder, predator-prey
     const int W = 2 * io->pp_env->vision + 1;
     if (W * W > PREP_MAX_WW || io->pp_env->B != cfg->B || ic3_pp_agents(*io->pp_env) != cfg->N) return IC3_E_RANGE;
@@ -264,7 +166,7 @@ static int tc_pass(const ic3_policy_cfg* cfg, const ic3_policy_packed* w, const 
     src.pps = *io->pp_state;
     if (int lrc = ic3_pp_layout_check(io->pp_env, cfg)) return lrc;
     if (src.table) {
-      IC3_LAUNCH_RC(ic3_launch_pdl(prep_kernel<XSRC_PP, true>, dim3(2 * ntiles_pad), dim3(PREP_THREADS), prep_T_bytes(cfg->N), s, *cfg, *io, img, src, PrepBwd{}));
+      prep_kernel<XSRC_PP, true><<<2 * ntiles, PREP_THREADS, prep_T_bytes(cfg->N), s>>>(*cfg, *io, img, src, PrepBwd{});
     } else {
       static bool cfgd = false;
       if (!cfgd) {
@@ -272,7 +174,7 @@ static int tc_pass(const ic3_policy_cfg* cfg, const ic3_policy_packed* w, const 
         if (e != cudaSuccess) return (int)e;
         cfgd = true;
       }
-      IC3_LAUNCH_RC(ic3_launch_pdl(prep_kernel<XSRC_PP, false>, dim3(2 * ntiles_pad), dim3(256), PREP_X_BYTES + prep_T_bytes(cfg->N), s, *cfg, *io, img, src, PrepBwd{}));
+      prep_kernel<XSRC_PP, false><<<2 * ntiles, 256, PREP_X_BYTES + prep_T_bytes(cfg->N), s>>>(*cfg, *io, img, src, PrepBwd{});
     }
   } else if (io->tj_env && io->tj_state) {       // fused index encoder, traffic junction
     const int W = 2 * io->tj_env->vision + 1;
@@ -282,7 +184,7 @@ static int tc_pass(const ic3_policy_cfg* cfg, const ic3_policy_packed* w, const 
     src.tjs = *io->tj_state;
     if (int lrc = ic3_tj_layout_check(io->tj_env, cfg)) return lrc;
     if (src.table) {
-      IC3_LAUNCH_RC(ic3_launch_pdl(prep_kernel<XSRC_TJ, true>, dim3(2 * ntiles_pad), dim3(PREP_THREADS), prep_T_bytes(cfg->N), s, *cfg, *io, img, src, PrepBwd{}));
+      prep_kernel<XSRC_TJ, true><<<2 * ntiles, PREP_THREADS, prep_T_bytes(cfg->N), s>>>(*cfg, *io, img, src, PrepBwd{});
     } else {
       static bool cfgd = false;
       if (!cfgd) {
@@ -290,37 +192,27 @@ static int tc_pass(const ic3_policy_cfg* cfg, const ic3_policy_packed* w, const 
         if (e != cudaSuccess) return (int)e;
         cfgd = true;
       }
-      IC3_LAUNCH_RC(ic3_launch_pdl(prep_kernel<XSRC_TJ, false>, dim3(2 * ntiles_pad), dim3(256), PREP_X_BYTES + prep_T_bytes(cfg->N), s, *cfg, *io, img, src, PrepBwd{}));
+      prep_kernel<XSRC_TJ, false><<<2 * ntiles, 256, PREP_X_BYTES + prep_T_bytes(cfg->N), s>>>(*cfg, *io, img, src, PrepBwd{});
     }
   } else {
     return IC3_E_NULL;
   }
+  IC3_LAUNCH_CHECK();
   prof_mark(1, s);
   const size_t smem = NSTAGE_P * STAGE_BYTES + 256 + TC_H * HEAD_PAD * sizeof(float) + 4 * TC_H * sizeof(float);
   int nout = 1;
   for (int k = 0; k < cfg->nheads; ++k) nout += cfg->head_dim[k];
   const bool fused_heads = nout <= HEAD_PAD;
   float* partial = fused_heads ? reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(io->workspace) +
-                                                           (size_t)ntiles_pad * TC_NCHUNK * A_CHUNK_BYTES)
+                                                           (size_t)ntiles * TC_NCHUNK * A_CHUNK_BYTES)
                                : nullptr;
-  int rc = IC3_E_RANGE;
-  if (tc_pair_mode()) rc = launch_lstm_pair(cfg, io, w, img, ntiles_pad, nout, partial, s);
-  else switch (tc_cluster_size()) {
-    case 1: rc = launch_lstm<1>(cfg, io, w, img, ntiles_pad, smem, nout, partial, s); break;
-    case 2: rc = launch_lstm<2>(cfg, io, w, img, ntiles_pad, smem, nout, partial, s); break;
-    case 4: rc = launch_lstm<4>(cfg, io, w, img, ntiles_pad, smem, nout, partial, s); break;
-    case 8: rc = launch_lstm<8>(cfg, io, w, img, ntiles_pad, smem, nout, partial, s); break;
-  }
+  const int rc = launch_lstm(cfg, io, w, img, ntiles, smem, nout, partial, s);
   if (rc) return rc;
   prof_mark(2, s);
   if (!last) return IC3_OK;                  // heads after the last comm pass only
-  if (fused_heads && io->defer_heads) {      // the env step kernel finishes the heads (ic3_rollout_io.head_partial)
-    prof_mark(3, s);
-    return IC3_OK;
-  }
   if (fused_heads) {
-    IC3_LAUNCH_RC(ic3_launch_pdl(heads_finish_kernel, dim3((unsigned)((R + 127) / 128)), dim3(128), 0, s, *cfg, *w, *io,
-                                 (const float*)partial));
+    heads_finish_kernel<<<(unsigned)((R + 127) / 128), 128, 0, s>>>(*cfg, *w, *io, partial);
+    IC3_LAUNCH_CHECK();
     prof_mark(3, s);
     return IC3_OK;
   }

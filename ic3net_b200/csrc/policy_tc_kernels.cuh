@@ -7,7 +7,6 @@
 #include <cstring>
 
 #include "ic3_common.cuh"
-#include "policy_heads.cuh"
 #include "policy_internal.h"
 #include "tc_common.cuh"
 
@@ -40,12 +39,6 @@ __host__ __device__ __forceinline__ size_t b_img_off(int nh, int k, int n, int p
 }
 
 constexpr size_t B_IMG_HALFS = (size_t)2 * TC_NCHUNK * B_CHUNK_BYTES / 2;   // one weight image, in halfs
-// pair layout: [nh][chunk][rank = n >> 7][hi,lo][kcore 4][ncore 16][8][8]
-__host__ __device__ __forceinline__ size_t b_img2_off(int nh, int k, int n, int part) {
-  const int c = k >> 5, kk = k & 31, rank = n >> 7, nn = n & 127;
-  return (((((((size_t)(nh * TC_NCHUNK + c) * 2 + rank) * 2 + part) * 4 + (kk >> 3)) * 16 + (nn >> 3)) * 8 + (nn & 7)) * 8) +
-         (kk & 7);
-}
 
 // ---- weight images (once per optimizer step) ------------------------------------------------
 __global__ void pack_tc_kernel(ic3_policy_params p, __half* __restrict__ img, float* __restrict__ bias_cat,
@@ -71,10 +64,6 @@ __global__ void pack_tc_kernel(ic3_policy_params p, __half* __restrict__ img, fl
     const int nh = col >> 8, n = col & 255;
     img[b_img_off(nh, k, n, 0)] = hi;
     img[b_img_off(nh, k, n, 1)] = lo;
-    // second copy for the cta_group::2 kernel: each CTA of a pair owns 128 of the 256 columns
-    __half* img2 = img + B_IMG_HALFS;
-    img2[b_img2_off(nh, k, n, 0)] = hi;
-    img2[b_img2_off(nh, k, n, 1)] = lo;
   }
   if (idx < 4 * H) {
     const int u = idx >> 2, g = idx & 3, row = g * H + u;
@@ -161,12 +150,10 @@ __global__ void __launch_bounds__(256) prep_kernel(ic3_policy_cfg cfg, ic3_polic
   const int R = cfg.B * N;
   const int tile = blockIdx.x >> 1, hb = blockIdx.x & 1;
   const int row0 = tile * TC_M + hb * PREP_ROWS;
-  ic3_pdl_trigger();
   if (TAB) {
     if (threadIdx.x < PREP_ROWS) s_mask[threadIdx.x] = 0u;
     __syncthreads();
   }
-  ic3_pdl_wait();      // h, masks, env state: written by the previous kernels of the step
   if (blockIdx.x == 0 && threadIdx.x == 0 && src.wflags && io.err && *src.wflags) atomicOr(io.err, *src.wflags);
   for (int w = threadIdx.x; w < PREP_ROWS + 64; w += blockDim.x) {
     const int row = row0 - 32 + w;
@@ -440,21 +427,6 @@ __device__ __forceinline__ float rcp_fast(float x) {
 }
 constexpr float LOG2E = 1.4426950408889634f;
 
-#ifdef IC3_TC_EXP_TRACE
-// Profiling experiment only (profiles/microbench/trace_lstm.py): CTA 0 timestamps its pipeline roles with
-// %globaltimer so that the overlap of operand stream, MMAs and epilogue can be read off directly.
-__device__ unsigned long long g_tc_trace[4][512];
-__device__ __forceinline__ void tc_trace(int role, int& idx) {
-  if (blockIdx.x == 0 && idx < 512) {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    g_tc_trace[role][idx++] = t;
-  }
-}
-#define TC_TRACE(role, idx) tc_trace(role, idx)
-#else
-#define TC_TRACE(role, idx)
-#endif
 // Gate biases pre-multiplied like the accumulator scale: (i, f, o) * -log2(e), g * -2 log2(e); [4H] in shared memory.
 __device__ __forceinline__ void load_scaled_bias(float* s_bias, const float* __restrict__ bias_cat) {
   for (int idx = threadIdx.x; idx < 4 * TC_H; idx += blockDim.x)
@@ -470,14 +442,6 @@ __device__ __forceinline__ void load_scaled_bias(float* s_bias, const float* __r
 __device__ __forceinline__ void lstm_cell4(const uint32_t (&v)[16], const float (&co)[4], const float* s_bias4,
                                            float (&cn)[4], float (&hn)[4]) {
   constexpr float SG = -INV_SCALE * LOG2E;
-#ifdef IC3_TC_EXP_SKIP_MATH   // profiling experiment only (profiles/microbench): epilogue without the SFU work
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    cn[j] = fmaf(__uint_as_float(v[4 * j + 1]), SG, co[j]) + __uint_as_float(v[4 * j]);
-    hn[j] = fmaf(__uint_as_float(v[4 * j + 2]), SG, s_bias4[4 * j]) + __uint_as_float(v[4 * j + 3]);
-  }
-  return;
-#endif
   constexpr float TMAX = 30.f;
   float go[4], bc[4];
 #pragma unroll
@@ -515,11 +479,11 @@ __device__ __forceinline__ void lstm_cell4(const uint32_t (&v)[16], const float 
 //                      overlaps the MMAs of item i+1
 // Work item = (128-row tile, 256-column half); item 2t and 2t+1 share the A tile (second read hits L2).
 constexpr int NSTAGE_P = 4;
-constexpr int HEAD_PAD = IC3_HEAD_PAD;   // outputs (value + action logits) the fused epilogue supports
+constexpr int HEAD_PAD = 8;          // outputs (value + action logits) the fused epilogue supports
 constexpr int EPI_WARPS = 16;        // 4 warps per TMEM lane quarter, 64 accumulator columns (16 hidden units) each
 constexpr int EPI_THREADS = EPI_WARPS * 32;
 constexpr int TC_P_THREADS = EPI_THREADS + 64;   // + producer warp + MMA warp
-constexpr int NSLOT = IC3_HEAD_NSLOT;   // partial-logit slots per row: (column half of the item) x (column quarter of the warp)
+constexpr int NSLOT = 8;             // partial-logit slots per row: (column half of the item) x (column quarter of the warp)
 
 // Two adjacent lanes (rows 2k, 2k+1 of the tile) hold 8 consecutive floats of their own row each (a = first 4,
 // b = last 4).  Written directly, every STG.128 of the warp touches 32 half-used 32-byte sectors; after one
@@ -532,17 +496,10 @@ __device__ __forceinline__ void pair_store8(float* pe, float* po, const float (&
   for (int j = 0; j < 4; ++j) r[j] = __shfl_xor_sync(IC3_FULL_MASK, odd ? a[j] : b[j], 1);
   const float4 x1 = odd ? make_float4(r[0], r[1], r[2], r[3]) : make_float4(a[0], a[1], a[2], a[3]);
   const float4 x2 = odd ? make_float4(b[0], b[1], b[2], b[3]) : make_float4(r[0], r[1], r[2], r[3]);
-#ifdef IC3_TC_EXP_SKIP_STORE   // profiling experiment only: keep the values live, store (almost) nothing
-  ev = ev && (x1.x + x1.y + x1.z + x1.w == 12345.678f);
-  ov = ov && (x2.x + x2.y + x2.z + x2.w == 12345.678f);
-#endif
   if (ev) *reinterpret_cast<float4*>(pe + (odd ? 4 : 0)) = x1;
   if (ov) *reinterpret_cast<float4*>(po + (odd ? 4 : 0)) = x2;
 }
 
-// One work item of an epilogue thread = (row of the tile, 16 hidden units): LSTM cell from the finished
-// accumulator, h'/c' stores, partial head logits.  `remote_release`: the accumulator barrier lives in the
-// leader CTA of the pair (cta_group::2 kernel).
 // Previous cell state of an epilogue thread's 16 hidden units (zero for a fresh episode).  Independent of the
 // MMAs, so the caller issues it before waiting for the accumulator.  (Prefetching it one whole item ahead was
 // measured: no gain -- the load is not on the critical path -- and the 16 extra live registers cost 4%.)
@@ -561,37 +518,20 @@ __device__ __forceinline__ void load_cold(const ic3_policy_cfg& cfg, const ic3_p
   }
 }
 
+// One work item of an epilogue thread = (row of the tile, 16 hidden units): LSTM cell from the finished
+// accumulator, h'/c' stores, partial head logits.
 __device__ __forceinline__ void epilogue_item(const ic3_policy_cfg& cfg, const ic3_policy_io& io, const float* s_bias,
                                               const float* s_hw, float* __restrict__ partial, uint32_t tmem_base,
                                               uint32_t bar_tfull, uint32_t bar_tempty, uint32_t li, int tile, int nh,
-                                              int quarter, int cq, int lane, const float4 (&cold)[4], bool& ok,
-                                              bool remote_release) {
+                                              int quarter, int cq, int lane, const float4 (&cold)[4], bool& ok) {
   const uint32_t acc = li & 1;
   const int R = cfg.B * cfg.N;
   const int row = tile * TC_M + quarter * 32 + lane;       // row parity == lane parity
   const bool odd = lane & 1;
   const bool inrange = row < R;
   const int ubase = nh * (TC_NH / 4) + cq * 16;
-#ifdef IC3_TC_EXP_TRACE
-  int tr = 4 * (int)li;
-  const bool tracer = quarter == 0 && cq == 0 && lane == 0;
-  if (tracer) TC_TRACE(2, tr);
-#endif
   if (ok) ok = mbar_wait(bar_tfull + 8 * acc, (li >> 1) & 1, io.err);
   tc_fence_after();
-#ifdef IC3_TC_EXP_TRACE
-  if (tracer) TC_TRACE(2, tr);
-#endif
-#ifdef IC3_TC_EXP_SKIP_EPI   // profiling experiment only: the epilogue just hands the accumulator back
-  tc_fence_before();
-  __syncwarp();
-  if (lane == 0) {
-    if (!remote_release) mbar_arrive(bar_tempty + 8 * acc);
-    else mbar_arrive_remote(bar_tempty + 8 * acc, 0);
-  }
-  if (cold[0].x == 12345.678f && partial) partial[row] = cold[1].y + cold[2].z + cold[3].w + s_bias[ubase] + s_hw[odd];
-  return;
-#endif
   const bool valid = ok && inrange;
   const int erow = row & ~1, orow = row | 1;
   const bool ev = ok && erow < R, ov = ok && orow < R;     // validity of the two rows this lane pair writes
@@ -629,14 +569,8 @@ __device__ __forceinline__ void epilogue_item(const ic3_policy_cfg& cfg, const i
     pair_store8(io.h_out + (size_t)erow * TC_H + u0, io.h_out + (size_t)orow * TC_H + u0, hn0, hn1, ev, ov, odd);
   }
   tc_fence_before();
-#ifdef IC3_TC_EXP_TRACE
-  if (tracer) TC_TRACE(2, tr);
-#endif
   __syncwarp();                              // every lane of the warp is done reading the accumulator:
-  if (lane == 0) {                           // one arrival per warp (remote arrivals on one barrier serialise)
-    if (!remote_release) mbar_arrive(bar_tempty + 8 * acc);
-    else mbar_arrive_remote(bar_tempty + 8 * acc, 0);        // ... on the leader's barrier
-  }
+  if (lane == 0) mbar_arrive(bar_tempty + 8 * acc);        // one arrival per warp
   if (partial) {                             // slot = (column half of the item, column quarter of the warp)
     const size_t so = (size_t)(nh * 4 + cq) * HEAD_PAD;
     const float pa[4] = {part[0], part[1], part[2], part[3]}, pb[4] = {part[4], part[5], part[6], part[7]};
@@ -645,10 +579,6 @@ __device__ __forceinline__ void epilogue_item(const ic3_policy_cfg& cfg, const i
   }
 }
 
-// CL = thread-block cluster size.  The CL CTAs of a cluster work on CL consecutive row tiles and the SAME
-// column half, so they consume identical weight (B) chunks: each CTA fetches 1/CL of every chunk and multicasts
-// it to all peers; a stage is recycled when the MMAs of ALL peers have released it (multicast commit).
-template <int CL>
 __global__ void __launch_bounds__(TC_P_THREADS, 1) lstm_tc_kernel(ic3_policy_cfg cfg, ic3_policy_io io,
                                                                  const __half* __restrict__ a_img,
                                                                  const __half* __restrict__ b_img,
@@ -662,18 +592,14 @@ __global__ void __launch_bounds__(TC_P_THREADS, 1) lstm_tc_kernel(ic3_policy_cfg
   // of its 32 hidden units into per-slot partial logits (partial != nullptr  <=>  nout <= 8)
   float* s_hw = reinterpret_cast<float*>(smem + NSTAGE_P * STAGE_BYTES + 256);
   float* s_bias = s_hw + TC_H * HEAD_PAD;
-  ic3_pdl_trigger();
   const uint32_t bar_full = smem_u32(bars), bar_empty = smem_u32(bars + NSTAGE_P);
   const uint32_t bar_tfull = smem_u32(bars + 2 * NSTAGE_P), bar_tempty = smem_u32(bars + 2 * NSTAGE_P + 2);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int rank = CL > 1 ? (int)cluster_ctarank() : 0;
-  const int cl = blockIdx.x / CL, ncl = gridDim.x / CL;     // this cluster / clusters in the grid
-  constexpr uint16_t CMASK = (uint16_t)((1u << CL) - 1u);
 
   if (threadIdx.x == 0) {
     for (int s = 0; s < NSTAGE_P; ++s) {
       mbar_init(bar_full + 8 * s, 1);
-      mbar_init(bar_empty + 8 * s, CL);        // one release from the MMA warp of every CTA in the cluster
+      mbar_init(bar_empty + 8 * s, 1);         // released by the MMA warp's commit
     }
     for (int a = 0; a < 2; ++a) {
       mbar_init(bar_tfull + 8 * a, 1);
@@ -686,9 +612,6 @@ __global__ void __launch_bounds__(TC_P_THREADS, 1) lstm_tc_kernel(ic3_policy_cfg
                  : "memory");
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
-  // barriers and TMEM are set up while the previous kernel (prep) drains; weights (they may have been re-packed by
-  // an earlier kernel of the stream) and the operand image are only touched from here on
-  ic3_pdl_wait();
   load_scaled_bias(s_bias, bias_cat);
   if (partial) {
     for (int idx = threadIdx.x; idx < TC_H * HEAD_PAD; idx += blockDim.x) {
@@ -698,7 +621,6 @@ __global__ void __launch_bounds__(TC_P_THREADS, 1) lstm_tc_kernel(ic3_policy_cfg
   }
   tc_fence_before();
   __syncthreads();
-  if (CL > 1) cluster_sync_all();              // peers' barriers are initialised before anything is multicast
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
@@ -707,10 +629,9 @@ __global__ void __launch_bounds__(TC_P_THREADS, 1) lstm_tc_kernel(ic3_policy_cfg
     static_assert(TC_NCHUNK % NSTAGE_P == 0, "stage index must be a function of the chunk index alone");
     uint32_t li = 0;
     bool ok = true;
-    [[maybe_unused]] int tr = 0;
     const uint32_t smem_base = smem_u32(smem);
-    for (int item = cl; item < nitems && ok; item += ncl, ++li) {
-      const int tile = (item >> 1) * CL + rank, nh = item & 1;
+    for (int item = blockIdx.x; item < nitems && ok; item += gridDim.x, ++li) {
+      const int tile = item >> 1, nh = item & 1;
       const unsigned char* a_src = reinterpret_cast<const unsigned char*>(a_img) + (size_t)tile * TC_NCHUNK * A_CHUNK_BYTES;
       const unsigned char* b_src = reinterpret_cast<const unsigned char*>(b_img) + (size_t)nh * TC_NCHUNK * B_CHUNK_BYTES;
       // TC_NCHUNK is a multiple of the ring depth: chunk c of every item uses stage c % NSTAGE_P, so the stage
@@ -720,23 +641,12 @@ __global__ void __launch_bounds__(TC_P_THREADS, 1) lstm_tc_kernel(ic3_policy_cfg
         if (!ok) break;
         const uint32_t s = c % NSTAGE_P;
         ok = mbar_wait(bar_empty + 8 * s, ((li * (TC_NCHUNK / NSTAGE_P) + c / NSTAGE_P) & 1) ^ 1, io.err);
-        if (c == 0 || c == TC_NCHUNK - 1) TC_TRACE(0, tr);
         const uint32_t dst = smem_base + s * STAGE_BYTES;
-#ifdef IC3_TC_EXP_SKIP_TMA   // profiling experiment only: pipeline without the operand stream
-        mbar_arrive(bar_full + 8 * s);
-        continue;
-#endif
         mbar_expect_tx(bar_full + 8 * s, STAGE_BYTES);
         bulk_g2s(dst, a_src + (size_t)c * (A_CHUNK_BYTES / 2), A_CHUNK_BYTES / 2, bar_full + 8 * s);                       // hi
         bulk_g2s(dst + A_CHUNK_BYTES / 2, a_src + A_TILE_HALFS + (size_t)c * (A_CHUNK_BYTES / 2), A_CHUNK_BYTES / 2,   // lo
                  bar_full + 8 * s);
-        if (CL == 1) {
-          bulk_g2s(dst + A_CHUNK_BYTES, b_src + (size_t)c * B_CHUNK_BYTES, B_CHUNK_BYTES, bar_full + 8 * s);
-        } else {      // my 1/CL slice of the weight chunk, delivered to every CTA of the cluster
-          constexpr uint32_t SL = B_CHUNK_BYTES / CL;
-          bulk_g2s_mc(dst + A_CHUNK_BYTES + rank * SL, b_src + (size_t)c * B_CHUNK_BYTES + (size_t)rank * SL, SL,
-                      bar_full + 8 * s, CMASK);
-        }
+        bulk_g2s(dst + A_CHUNK_BYTES, b_src + (size_t)c * B_CHUNK_BYTES, B_CHUNK_BYTES, bar_full + 8 * s);
       }
     }
   } else if (warp == EPI_WARPS + 1 && lane == 0) {
@@ -745,15 +655,13 @@ __global__ void __launch_bounds__(TC_P_THREADS, 1) lstm_tc_kernel(ic3_policy_cfg
     const uint32_t idesc = (1u << 4) | ((uint32_t)(TC_NH >> 3) << 17) | ((uint32_t)(TC_M >> 4) << 24);
     uint32_t li = 0;
     bool ok = true;
-    [[maybe_unused]] int tr = 0;
     // descriptors of stage 0 / k-step 0; every other one is + (byte offset >> 4) in the address field.
     // A: kcore block = 16 rcores x 128 B = 2048 B; B: 32 ncores x 128 B = 4096 B; lo half follows hi half
     const uint64_t dA = make_desc(smem_u32(smem), 2048, 128), dB = make_desc(smem_u32(smem) + A_CHUNK_BYTES, 4096, 128);
-    for (int item = cl; item < nitems && ok; item += ncl, ++li) {
+    for (int item = blockIdx.x; item < nitems && ok; item += gridDim.x, ++li) {
       const uint32_t acc = li & 1;
       ok = mbar_wait(bar_tempty + 8 * acc, ((li >> 1) & 1) ^ 1, io.err);   // epilogue drained this accumulator
       tc_fence_after();
-      TC_TRACE(1, tr);
       const uint32_t tmem_d = tmem_base + acc * TC_NH;
 #pragma unroll
       for (int c = 0; c < TC_NCHUNK; ++c) {
@@ -761,21 +669,17 @@ __global__ void __launch_bounds__(TC_P_THREADS, 1) lstm_tc_kernel(ic3_policy_cfg
         const uint32_t s = c % NSTAGE_P;
         ok = mbar_wait(bar_full + 8 * s, (li * (TC_NCHUNK / NSTAGE_P) + c / NSTAGE_P) & 1, io.err);
         tc_fence_after();
-        if (c == 0 || c == TC_NCHUNK - 1) TC_TRACE(1, tr);
 #pragma unroll
         for (int ks = 0; ks < TC_KC / 16; ++ks) {
           const uint64_t da_hi = dA + ((s * STAGE_BYTES + ks * 4096) >> 4);
           const uint64_t da_lo = dA + ((s * STAGE_BYTES + A_CHUNK_BYTES / 2 + ks * 4096) >> 4);
           const uint64_t db_hi = dB + ((s * STAGE_BYTES + ks * 8192) >> 4);
           const uint64_t db_lo = dB + ((s * STAGE_BYTES + B_CHUNK_BYTES / 2 + ks * 8192) >> 4);
-#ifndef IC3_TC_EXP_SKIP_MMA   // profiling experiment only: pipeline without the tensor work
           tc_mma_f16(tmem_d, da_hi, db_hi, idesc, (c | ks) != 0);
           tc_mma_f16(tmem_d, da_lo, db_hi, idesc, 1);
           tc_mma_f16(tmem_d, da_hi, db_lo, idesc, 1);
-#endif
         }
-        if (CL == 1) tc_commit(bar_empty + 8 * s);      // frees the stage when these MMAs have read it
-        else tc_commit_mc(bar_empty + 8 * s, CMASK);    // ... in every CTA of the cluster
+        tc_commit(bar_empty + 8 * s);      // frees the stage when these MMAs have read it
       }
       tc_commit(bar_tfull + 8 * acc);      // accumulator complete
     }
@@ -784,17 +688,15 @@ __global__ void __launch_bounds__(TC_P_THREADS, 1) lstm_tc_kernel(ic3_policy_cfg
     const int quarter = warp & 3, cq = warp >> 2;
     uint32_t li = 0;
     bool ok = true;
-    for (int item = cl; item < nitems; item += ncl, ++li) {
-      const int tile = (item >> 1) * CL + rank, nh = item & 1;
+    for (int item = blockIdx.x; item < nitems; item += gridDim.x, ++li) {
+      const int tile = item >> 1, nh = item & 1;
       float4 cold[4];         // issued before the accumulator wait: overlaps the MMAs of this item
       load_cold(cfg, io, tile, nh, quarter, cq, lane, cold);
-      epilogue_item(cfg, io, s_bias, s_hw, partial, tmem_base, bar_tfull, bar_tempty, li, tile, nh, quarter, cq, lane, cold, ok,
-                    false);
+      epilogue_item(cfg, io, s_bias, s_hw, partial, tmem_base, bar_tfull, bar_tempty, li, tile, nh, quarter, cq, lane, cold, ok);
     }
   }
   tc_fence_before();
   __syncthreads();
-  if (CL > 1) cluster_sync_all();              // no peer may still multicast into / arrive on this CTA
   if (warp == EPI_WARPS) {
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
   }
@@ -880,170 +782,77 @@ __global__ void __launch_bounds__(256) heads_kernel(ic3_policy_cfg cfg, ic3_poli
   }
 }
 
-// cta_group::2 version: a CTA pair (cluster of 2) computes a 256-row x 256-column item with ONE 2-SM MMA stream.
-// Each CTA stages its own 128 A rows (16 KB / chunk) and only HALF of the weight chunk (16 KB instead of 32 KB),
-// so the per-SM operand stream drops by a third and the ring holds 6 stages.  Protocol (as in CUTLASS 2-SM kernels):
-// both CTAs allocate TMEM with cta_group::2; the leader (rank 0) issues tcgen05.mma.cta_group::2 once its own stage
-// AND the peer's stage have landed (the peer relays its mbarrier phase with a remote arrive); stage and accumulator
-// hand-offs are multicast commits; both epilogues release the accumulator on the leader's barrier.
-constexpr int PAIR_STAGE_BYTES = A_CHUNK_BYTES + B_CHUNK_BYTES / 2;   // 32 KB
-constexpr int PAIR_NSTAGE = 6;
-__global__ void __launch_bounds__(TC_P_THREADS, 1) lstm_tc_pair_kernel(ic3_policy_cfg cfg, ic3_policy_io io,
-                                                                 const __half* __restrict__ a_img,
-                                                                 const __half* __restrict__ b_img,
-                                                                 const float* __restrict__ bias_cat, int nitems,
-                                                                 const float* __restrict__ head_w, int nout,
-                                                                 float* __restrict__ partial) {
-  extern __shared__ __align__(1024) unsigned char smem[];
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + PAIR_NSTAGE * PAIR_STAGE_BYTES);
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 30);
-  // head weights, unit-major [128][8] (zero padded): the epilogue folds value/action-head dot products
-  // of its 32 hidden units into per-slot partial logits (partial != nullptr  <=>  nout <= 8)
-  float* s_hw = reinterpret_cast<float*>(smem + PAIR_NSTAGE * PAIR_STAGE_BYTES + 256);
-  float* s_bias = s_hw + TC_H * HEAD_PAD;
-  ic3_pdl_trigger();
-  const uint32_t bar_full = smem_u32(bars), bar_empty = smem_u32(bars + PAIR_NSTAGE);
-  const uint32_t bar_pfull = smem_u32(bars + 2 * PAIR_NSTAGE);      // leader: "the peer's stage has landed"
-  const uint32_t bar_tfull = smem_u32(bars + 3 * PAIR_NSTAGE), bar_tempty = smem_u32(bars + 3 * PAIR_NSTAGE + 2);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  constexpr int CL = 2;
-  const int rank = (int)cluster_ctarank();
-  const int cl = blockIdx.x / CL, ncl = gridDim.x / CL;     // this pair / pairs in the grid
-  constexpr uint16_t CMASK = 3;
+// Finishing the heads from the per-slot partial logits of the LSTM epilogue (fixed summation order -> deterministic):
+// value, log-softmax per head, inverse-CDF sampling of ONE agent row by ONE thread.
+struct HeadsFinish {
+  const float* partial;   // [R][NSLOT][HEAD_PAD]
+  const float* head_b;    // [1 + sum(na)]
+  int nheads;
+  int head_dim[IC3_MAX_HEADS];
+  uint64_t seed;
+  uint32_t env_id0;
+  const uint32_t* tick;   // [B] or NULL
+  const uint32_t* draws;  // [R, nheads] or NULL
+  float* value;           // [R]
+  float* logp;            // [R, sum(na)]
+  int32_t* action;        // [R, nheads] or NULL (no sampling)
+};
 
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < PAIR_NSTAGE; ++s) {
-      mbar_init(bar_full + 8 * s, 1);
-      mbar_init(bar_empty + 8 * s, 1);         // the leader's multicast commit arrives once in each CTA
-      mbar_init(bar_pfull + 8 * s, 1);
-    }
-    for (int a = 0; a < 2; ++a) {
-      mbar_init(bar_tfull + 8 * a, 1);
-      mbar_init(bar_tempty + 8 * a, 2 * EPI_WARPS);     // one arrival per epilogue warp of both CTAs (leader's barrier)
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == EPI_WARPS) {   // all 512 TMEM columns: two 128-lane x 256-column fp32 accumulators
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  ic3_pdl_wait();
-  load_scaled_bias(s_bias, bias_cat);
-  if (partial) {
-    for (int idx = threadIdx.x; idx < TC_H * HEAD_PAD; idx += blockDim.x) {
-      const int u = idx / HEAD_PAD, o = idx - u * HEAD_PAD;
-      s_hw[idx] = o < nout ? __ldg(head_w + (size_t)o * TC_H + u) : 0.f;
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();                          // the peer's barriers are initialised before any remote arrive / commit
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == EPI_WARPS && lane == 0) {
-    // ===== producer =====
-    static_assert(TC_NCHUNK % PAIR_NSTAGE == 0, "stage index must be a function of the chunk index alone");
-    uint32_t li = 0;
-    bool ok = true;
-    [[maybe_unused]] int tr = 0;
-    const uint32_t smem_base = smem_u32(smem);
-    for (int item = cl; item < nitems && ok; item += ncl, ++li) {
-      const int tile = (item >> 1) * CL + rank, nh = item & 1;
-      const unsigned char* a_src = reinterpret_cast<const unsigned char*>(a_img) + (size_t)tile * TC_NCHUNK * A_CHUNK_BYTES;
-      // pair image: [nh][chunk][rank][16 KB]
-      const unsigned char* b_src = reinterpret_cast<const unsigned char*>(b_img) + (size_t)nh * TC_NCHUNK * B_CHUNK_BYTES +
-                                   (size_t)rank * (B_CHUNK_BYTES / 2);
+__device__ __forceinline__ void heads_finish_row(const HeadsFinish& f, long row, int e, int i) {
+  float logit[HEAD_PAD];
+  const float4* p4 = reinterpret_cast<const float4*>(f.partial + (size_t)row * NSLOT * HEAD_PAD);
+  {
+    float4 a = p4[0], b = p4[1];
 #pragma unroll
-      for (int c = 0; c < TC_NCHUNK; ++c) {       // stage index = c % PAIR_NSTAGE: compile-time constant
-        if (!ok) break;
-        const uint32_t s = c % PAIR_NSTAGE;
-        ok = mbar_wait(bar_empty + 8 * s, ((li * (TC_NCHUNK / PAIR_NSTAGE) + c / PAIR_NSTAGE) & 1) ^ 1, io.err);
-        if (c == 0 || c == TC_NCHUNK - 1) TC_TRACE(0, tr);
-        const uint32_t dst = smem_base + s * PAIR_STAGE_BYTES;
-#ifdef IC3_TC_EXP_SKIP_TMA
-        mbar_arrive(bar_full + 8 * s);
-        continue;
-#endif
-        mbar_expect_tx(bar_full + 8 * s, PAIR_STAGE_BYTES);
-        bulk_g2s(dst, a_src + (size_t)c * (A_CHUNK_BYTES / 2), A_CHUNK_BYTES / 2, bar_full + 8 * s);                       // hi
-        bulk_g2s(dst + A_CHUNK_BYTES / 2, a_src + A_TILE_HALFS + (size_t)c * (A_CHUNK_BYTES / 2), A_CHUNK_BYTES / 2,   // lo
-                 bar_full + 8 * s);
-        bulk_g2s(dst + A_CHUNK_BYTES, b_src + (size_t)c * B_CHUNK_BYTES, B_CHUNK_BYTES / 2, bar_full + 8 * s);
-      }
+    for (int sl = 1; sl < NSLOT; ++sl) {
+      const float4 c = p4[2 * sl], d = p4[2 * sl + 1];
+      a.x += c.x; a.y += c.y; a.z += c.z; a.w += c.w;
+      b.x += d.x; b.y += d.y; b.z += d.z; b.w += d.w;
     }
-  } else if (warp == EPI_WARPS + 1 && lane == 0) {
-    // ===== MMA issuer =====
-    // instruction descriptor: D = f32, A = B = f16, K-major both, N = 256, M = 256 over the CTA pair
-    const uint32_t idesc = (1u << 4) | ((uint32_t)(TC_NH >> 3) << 17) | ((uint32_t)((2 * TC_M) >> 4) << 24);
-    uint32_t li = 0;
-    bool ok = true;
-    if (rank != 0) {
-      // peer: relay "my stage has landed" to the leader, chunk by chunk
-      for (int item = cl; item < nitems && ok; item += ncl, ++li) {
+    logit[0] = a.x; logit[1] = a.y; logit[2] = a.z; logit[3] = a.w;
+    logit[4] = b.x; logit[5] = b.y; logit[6] = b.z; logit[7] = b.w;
+  }
+  int atot = 0;
+  for (int k = 0; k < f.nheads; ++k) atot += f.head_dim[k];
 #pragma unroll
-        for (int c = 0; c < TC_NCHUNK; ++c) {
-          if (!ok) break;
-          const uint32_t s = c % PAIR_NSTAGE;
-          ok = mbar_wait(bar_full + 8 * s, (li * (TC_NCHUNK / PAIR_NSTAGE) + c / PAIR_NSTAGE) & 1, io.err);
-          mbar_arrive_remote(bar_pfull + 8 * s, 0);
+  for (int o = 0; o < HEAD_PAD; ++o) logit[o] += (o < 1 + atot) ? __ldg(f.head_b + o) : 0.f;
+  f.value[row] = logit[0];
+  const bool do_sample = f.action != nullptr;
+  uint4 d24 = make_uint4(0, 0, 0, 0);
+  if (do_sample && !f.draws)
+    d24 = ic3_draw24(f.seed, f.env_id0 + (uint32_t)e, f.tick ? f.tick[e] : 0u, IC3_STREAM_ACTION, (uint32_t)i);
+  int off = 1;
+  for (int k = 0; k < f.nheads; ++k) {
+    const int na = f.head_dim[k];
+    float m = -INFINITY;
+#pragma unroll
+    for (int o = 1; o < HEAD_PAD; ++o)
+      if (o >= off && o < off + na) m = fmaxf(m, logit[o]);
+    float ssum = 0.f;
+#pragma unroll
+    for (int o = 1; o < HEAD_PAD; ++o)
+      if (o >= off && o < off + na) ssum += expf(logit[o] - m);
+    const float lse = m + logf(ssum);
+    uint32_t u24 = 0;
+    if (do_sample) u24 = f.draws ? f.draws[(size_t)row * f.nheads + k] : ic3_word(d24, k);
+    const float u = (float)u24 * 5.9604644775390625e-08f;
+    float cdf = 0.f;
+    int act = na - 1;
+    bool found = false;
+#pragma unroll
+    for (int o = 1; o < HEAD_PAD; ++o) {
+      if (o >= off && o < off + na) {
+        const float lp = logit[o] - lse;
+        f.logp[(size_t)row * atot + (o - 1)] = lp;
+        cdf += expf(lp);
+        if (!found && cdf > u) {
+          act = o - off;
+          found = true;
         }
       }
     }
-    [[maybe_unused]] int tr = 0, tr3 = 0;
-    // per CTA: A 128 rows (kcore block 2048 B), B 128 of the 256 columns (kcore block 16 ncores x 128 B = 2048 B)
-    const uint64_t dA = make_desc(smem_u32(smem), 2048, 128), dB = make_desc(smem_u32(smem) + A_CHUNK_BYTES, 2048, 128);
-    for (int item = cl; rank == 0 && item < nitems && ok; item += ncl, ++li) {
-      const uint32_t acc = li & 1;
-      ok = mbar_wait(bar_tempty + 8 * acc, ((li >> 1) & 1) ^ 1, io.err);   // both epilogues drained this accumulator
-      tc_fence_after();
-      TC_TRACE(1, tr);
-      const uint32_t tmem_d = tmem_base + acc * TC_NH;
-#pragma unroll
-      for (int c = 0; c < TC_NCHUNK; ++c) {
-        if (!ok) break;
-        const uint32_t s = c % PAIR_NSTAGE;
-        const uint32_t ph = (li * (TC_NCHUNK / PAIR_NSTAGE) + c / PAIR_NSTAGE) & 1;
-        ok = mbar_wait(bar_full + 8 * s, ph, io.err);
-        if (c == 0 || c == TC_NCHUNK - 1) TC_TRACE(3, tr3);          // own stage landed
-        if (ok) ok = mbar_wait(bar_pfull + 8 * s, ph, io.err);
-        tc_fence_after();
-        if (c == 0 || c == TC_NCHUNK - 1) TC_TRACE(1, tr);           // ... and the peer's
-#pragma unroll
-        for (int ks = 0; ks < TC_KC / 16; ++ks) {
-          const uint64_t da_hi = dA + ((s * PAIR_STAGE_BYTES + ks * 4096) >> 4);
-          const uint64_t da_lo = dA + ((s * PAIR_STAGE_BYTES + A_CHUNK_BYTES / 2 + ks * 4096) >> 4);
-          const uint64_t db_hi = dB + ((s * PAIR_STAGE_BYTES + ks * 4096) >> 4);
-          const uint64_t db_lo = dB + ((s * PAIR_STAGE_BYTES + B_CHUNK_BYTES / 4 + ks * 4096) >> 4);
-#ifndef IC3_TC_EXP_SKIP_MMA
-          tc_mma2_f16(tmem_d, da_hi, db_hi, idesc, (c | ks) != 0);
-          tc_mma2_f16(tmem_d, da_lo, db_hi, idesc, 1);
-          tc_mma2_f16(tmem_d, da_hi, db_lo, idesc, 1);
-#endif
-        }
-        tc_commit2_mc(bar_empty + 8 * s, CMASK);    // frees the stage in both CTAs when these MMAs have read it
-      }
-      tc_commit2_mc(bar_tfull + 8 * acc, CMASK);    // accumulator complete, in both CTAs
-    }
-  } else if (warp < EPI_WARPS) {
-    // ===== epilogue: thread = (row of the tile, 16 hidden units) =====
-    const int quarter = warp & 3, cq = warp >> 2;
-    uint32_t li = 0;
-    bool ok = true;
-    for (int item = cl; item < nitems; item += ncl, ++li) {
-      const int tile = (item >> 1) * CL + rank, nh = item & 1;
-      float4 cold[4];         // issued before the accumulator wait: overlaps the MMAs of this item
-      load_cold(cfg, io, tile, nh, quarter, cq, lane, cold);
-      epilogue_item(cfg, io, s_bias, s_hw, partial, tmem_base, bar_tfull, bar_tempty, li, tile, nh, quarter, cq, lane, cold, ok,
-                    rank != 0);
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();                          // the peer may still read this CTA's smem / arrive on its barriers
-  if (warp == EPI_WARPS) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
+    if (do_sample) f.action[(size_t)row * f.nheads + k] = act;
+    off += na;
   }
 }
 
@@ -1051,8 +860,6 @@ __global__ void __launch_bounds__(TC_P_THREADS, 1) lstm_tc_pair_kernel(ic3_polic
 // value, log-softmax per head, inverse-CDF sampling.  One thread per agent row.
 __global__ void __launch_bounds__(128) heads_finish_kernel(ic3_policy_cfg cfg, ic3_policy_packed w, ic3_policy_io io,
                                                             const float* __restrict__ partial) {
-  ic3_pdl_trigger();
-  ic3_pdl_wait();      // the partial logits come from the LSTM kernel
   const long row = (long)blockIdx.x * blockDim.x + threadIdx.x;
   if (row >= (long)cfg.B * cfg.N) return;
   HeadsFinish f;
@@ -1062,7 +869,7 @@ __global__ void __launch_bounds__(128) heads_finish_kernel(ic3_policy_cfg cfg, i
   f.seed = cfg.seed; f.env_id0 = cfg.env_id0; f.tick = io.tick; f.draws = io.draws;
   f.value = io.value; f.logp = io.logp; f.action = io.action;
   const int e = (int)(row / cfg.N), i = (int)(row - (long)e * cfg.N);
-  heads_finish_row(f, row, e, i, nullptr);
+  heads_finish_row(f, row, e, i);
 }
 
 }  // namespace

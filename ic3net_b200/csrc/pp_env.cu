@@ -4,6 +4,7 @@
 // done [B] u8.  With cfg.enemy_comm the prey is agent row N of act / reward / obs (NA = N + 1 rows per env).  One CTA per environment; warp 0 owns the integer state (lane = agent,
 // reductions are ballots), all warps stream the observation block of the env:
 // [N * W*W cells][V] floats, contiguous, written once with 16-byte evict-first stores.
+#include <algorithm>
 #include <cstring>
 
 #include "ic3_common.cuh"
@@ -116,8 +117,6 @@ template <bool VEC4>
 __global__ void pp_step_kernel(PPArgs a, const int32_t* __restrict__ act, int act_stride,
                                float* __restrict__ reward, float* __restrict__ obs, int32_t* err,
                                RolloutOpt r, int do_step, int keep_l2) {
-  ic3_pdl_trigger();
-  ic3_pdl_wait();      // everything below reads state / actions written by the previous kernel of the step
   extern __shared__ uint32_t s_cell[];
   __shared__ int s_r[IC3_MAX_AGENTS + 1], s_c[IC3_MAX_AGENTS + 1];
   const int N = a.cfg.N, D = a.cfg.dim;
@@ -141,8 +140,7 @@ __global__ void pp_step_kernel(PPArgs a, const int32_t* __restrict__ act, int ac
         if (lane == 0) atomicOr(err, IC3_ERR_EPISODE_DONE);
       } else {
         int av = 4;
-        if (r.has && r.io.head_partial) av = ic3_rollout_heads(r.io, a.cfg.seed, a.cfg.env_id0, a.st.tick, e, NA, lane);
-        else if (lane < NA) av = act[((size_t)e * NA + lane) * act_stride];
+        if (lane < NA) av = act[((size_t)e * NA + lane) * act_stride];
         if (lane >= NA) av = 4;
         if (lane < NA && (av < 0 || av > a.cfg.naction)) atomicOr(err, IC3_ERR_BAD_ACTION);  // :137 (sic, <=)
         if (lane < N && !rch) {  // _take_action :212-252: every move is a clamped move
@@ -225,6 +223,23 @@ int pp_check(const ic3_pp_cfg* cfg, const ic3_pp_state* st) {
   return IC3_OK;
 }
 
+// Residency bound of the observation-writing launch (one 256-thread CTA per env): at most 4 CTAs per SM.  The kernel's
+// 46-48 registers would let 5 CTAs share an SM, and the observation write is then slower: on B200 (predator-prey hard,
+// 8192 envs, 1000 W) 0.190 ms at 5 CTAs/SM against 0.184 ms at 4.  Requesting more than a fifth of the SM's shared
+// memory per CTA (dynamic shared memory, unused beyond the kernel's own cell buffer) keeps the fifth CTA out.
+constexpr int PP_OBS_CTAS_PER_SM = 4;
+size_t pp_obs_smem_floor() {
+  static size_t floor = 0;
+  if (floor == 0) {
+    int dev = 0, per_sm = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&per_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, dev);
+    floor = (size_t)per_sm / (PP_OBS_CTAS_PER_SM + 1) + 1;
+    if (floor > 48 * 1024) floor = 48 * 1024;      // the default dynamic shared-memory limit of a launch
+  }
+  return floor;
+}
+
 int pp_launch(const ic3_pp_cfg* cfg, const ic3_pp_state* st, const int32_t* act, int act_stride,
               float* reward, float* obs, int32_t* err, const ic3_rollout_io* r, int do_step,
               cudaStream_t s) {
@@ -232,19 +247,16 @@ int pp_launch(const ic3_pp_cfg* cfg, const ic3_pp_state* st, const int32_t* act,
   const int W = 2 * cfg->vision + 1;
   const int V = cfg->dim * cfg->dim + 4;
   const int NA = ic3_pp_agents(*cfg);
-  const size_t smem = obs ? (size_t)NA * W * W * sizeof(uint32_t) : 0;
+  const size_t smem = obs ? std::max((size_t)NA * W * W * sizeof(uint32_t), pp_obs_smem_floor()) : 0;
   const int threads = obs ? 256 : 32 * IC3_ENV_WARPS;
   const int grid = obs ? cfg->B : (cfg->B + IC3_ENV_WARPS - 1) / IC3_ENV_WARPS;
   const bool vec4 = (V % 4 == 0) && ((reinterpret_cast<uintptr_t>(obs) & 15) == 0);
   RolloutOpt ro = make_rollout_opt(r);
   // small observation batches stay in L2 for the encoder that follows (see IC3_OBS_L2_KEEP_BYTES)
   const int keep = obs && (size_t)cfg->B * NA * W * W * V * sizeof(float) <= IC3_OBS_L2_KEEP_BYTES;
-  if (vec4)
-    IC3_LAUNCH_RC(ic3_launch_pdl(pp_step_kernel<true>, dim3(grid), dim3(threads), smem, s, a, act, act_stride, reward, obs,
-                                 err, ro, do_step, keep));
-  else
-    IC3_LAUNCH_RC(ic3_launch_pdl(pp_step_kernel<false>, dim3(grid), dim3(threads), smem, s, a, act, act_stride, reward, obs,
-                                 err, ro, do_step, keep));
+  if (vec4) pp_step_kernel<true><<<grid, threads, smem, s>>>(a, act, act_stride, reward, obs, err, ro, do_step, keep);
+  else pp_step_kernel<false><<<grid, threads, smem, s>>>(a, act, act_stride, reward, obs, err, ro, do_step, keep);
+  IC3_LAUNCH_CHECK();
   return IC3_OK;
 }
 

@@ -2,7 +2,6 @@
 // the warp that owns one environment (lane = agent) right after the env step.
 #pragma once
 #include "ic3_common.cuh"
-#include "policy_heads.cuh"
 
 struct RolloutOpt {
   int has;            // 0: plain gym semantics (ic3_rollout_io* was NULL)
@@ -90,20 +89,4 @@ __device__ __forceinline__ void ic3_rollout_snapshot(const ic3_rollout_io& r, in
     if (r.snap_fresh) r.snap_fresh[(size_t)t1 * B + e] = r.fresh[e];
     if (r.snap_tep) r.snap_tep[(size_t)t1 * B + e] = r.t_ep[e];
   }
-}
-
-// Fused policy heads (ic3_rollout_io.head_partial): lane = agent finishes its row and returns the env action (head 0).
-__device__ __forceinline__ int ic3_rollout_heads(const ic3_rollout_io& r, uint64_t seed, uint32_t env_id0,
-                                                 const uint32_t* tick, int e, int N, int lane) {
-  int first = 0;
-  if (lane < N) {
-    HeadsFinish f;
-    f.partial = r.head_partial; f.head_b = r.head_b; f.nheads = r.nheads;
-#pragma unroll
-    for (int k = 0; k < IC3_MAX_HEADS; ++k) f.head_dim[k] = r.head_dim[k];
-    f.seed = seed; f.env_id0 = env_id0; f.tick = tick; f.draws = nullptr;
-    f.value = r.head_value; f.logp = r.head_logp; f.action = const_cast<int32_t*>(r.action);
-    heads_finish_row(f, (long)e * N + lane, e, lane, &first);
-  }
-  return first;
 }

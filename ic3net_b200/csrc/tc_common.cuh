@@ -64,57 +64,10 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
                "l"(src), "r"(bytes), "r"(bar)
                : "memory");
 }
-// multicast variant: the bytes land at the same shared-memory offset of every CTA in `mask`, and complete_tx
-// is signalled on the mbarrier at the same offset of each destination CTA
-__device__ __forceinline__ void bulk_g2s_mc(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::"r"(dst),
-      "l"(src), "r"(bytes), "r"(bar), "h"(mask)
-      : "memory");
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-// arrive on the mbarrier at the same shared-memory offset of CTA `cta` of this cluster
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t bar, uint32_t cta) {
-  asm volatile(
-      "{\n\t.reg .b32 ra;\n\t"
-      "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-      "mbarrier.arrive.shared::cluster.b64 _, [ra];\n\t}" ::"r"(bar),
-      "r"(cta)
-      : "memory");
-}
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-// same, arriving on the mbarrier at this offset in every CTA of `mask` (stage release across a cluster)
-__device__ __forceinline__ void tc_commit_mc(uint32_t bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-               "h"(mask)
-               : "memory");
-}
-// 2-SM forms: the MMA spans the TMEM / shared memory of both CTAs of a pair (M = 256), issued by the leader
-__device__ __forceinline__ void tc_commit2_mc(uint32_t bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar),
-               "h"(mask)
-               : "memory");
-}
-__device__ __forceinline__ void tc_mma2_f16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
-                                            uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
 }
 // D[tmem] (+)= A[smem] . B[smem]^T, kind::f16 (fp16 inputs, fp32 accumulate), one CTA
 __device__ __forceinline__ void tc_mma_f16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,

@@ -90,8 +90,6 @@ __device__ __forceinline__ void tj_write_obs(const ic3_tj_cfg& cfg, const int* s
 __global__ void tj_step_kernel(TJArgs a, const int32_t* __restrict__ act, int act_stride,
                                const uint32_t* __restrict__ draws, float* __restrict__ reward,
                                float* __restrict__ obs, int32_t* err, RolloutOpt r, int do_step, int keep_l2) {
-  ic3_pdl_trigger();
-  ic3_pdl_wait();      // everything below reads state / actions written by the previous kernel of the step
   extern __shared__ uint32_t s_cell[];
   __shared__ int s_r[IC3_MAX_AGENTS], s_c[IC3_MAX_AGENTS], s_alive[IC3_MAX_AGENTS], s_rid[IC3_MAX_AGENTS],
       s_lact[IC3_MAX_AGENTS];
@@ -118,8 +116,7 @@ __global__ void tj_step_kernel(TJArgs a, const int32_t* __restrict__ act, int ac
       // ---- _take_action :540-581 ----
       int completed = 0;
       int av = 1;
-      if (r.has && r.io.head_partial) av = ic3_rollout_heads(r.io, cfg.seed, cfg.env_id0, a.st.tick, e, N, lane);
-      else if (lane < N) av = act[i * act_stride];
+      if (lane < N) av = act[i * act_stride];
       if (lane >= N) av = 1;
       if (lane < N && (av < 0 || av > 2)) atomicOr(err, IC3_ERR_BAD_ACTION);  // :228 (sic, <=)
       if (lane < N && alive) {
@@ -268,8 +265,8 @@ int tj_launch(const ic3_tj_cfg* cfg, const ic3_tj_state* st, const int32_t* act,
   const int grid = obs ? cfg->B : (cfg->B + IC3_ENV_WARPS - 1) / IC3_ENV_WARPS;
   RolloutOpt ro = make_rollout_opt(r);
   const int keep = obs && (size_t)cfg->B * cfg->N * (2 + W * W * cfg->vocab) * sizeof(float) <= IC3_OBS_L2_KEEP_BYTES;
-  IC3_LAUNCH_RC(ic3_launch_pdl(tj_step_kernel, dim3(grid), dim3(threads), smem, s, a, act, act_stride, draws, reward, obs, err,
-                               ro, do_step, keep));
+  tj_step_kernel<<<grid, threads, smem, s>>>(a, act, act_stride, draws, reward, obs, err, ro, do_step, keep);
+  IC3_LAUNCH_CHECK();
   return IC3_OK;
 }
 

@@ -248,18 +248,6 @@ class Trainer(object):
             src = dict(tj_env=C.addressof(e.cfg), tj_state=C.addressof(e.state)) if self.is_tj else \
                 dict(pp_env=C.addressof(e.cfg), pp_state=C.addressof(e.state))
             src['x_table'] = _lib.ptr(self._encoder_table(cfg, w))
-        # Option (args.fuse_heads, default off): on the tensor-core path with <= 7 action logits the env step kernel can
-        # finish the policy heads (value, log-softmax, sampling) from the LSTM epilogue's partial logits -- one launch
-        # less per lock-step iteration.  Measured on B200 (PP hard, 8192 envs): index step 0.172 ms fused vs 0.166 ms with
-        # the separate heads_finish kernel -- one 32-thread CTA per env hides the 64 partial-logit loads of a row worse
-        # than the thread-per-row kernel at full occupancy -- so the separate kernel stays the default.
-        fuse_heads = (net.policy_impl == 'tc' and 1 + sum(args.naction_heads) <= 8 and ws is not None
-                      and bool(getattr(args, 'fuse_heads', False)))
-        heads_kw = {}
-        if fuse_heads:
-            hd = (C.c_int32 * _lib.MAX_HEADS)(*(list(args.naction_heads) + [0] * (_lib.MAX_HEADS - nh)))
-            heads_kw = dict(head_partial=lib.ic3_policy_partial_ptr(C.byref(cfg), ws.data_ptr()),
-                            head_b=net._bufs['head_b'].data_ptr(), head_dim=hd)
         snap = {}
         if rec:
             snap = dict(snap_T=T, snap_fresh=b['s_fresh'].data_ptr(), snap_comm=b['s_comm'].data_ptr(),
@@ -311,14 +299,12 @@ class Trainer(object):
                                fresh=b['fresh'].data_ptr(), tick=e.tick.data_ptr(), draws=None,
                                h_out=hout.data_ptr(), c_out=cout.data_ptr(), value=b['value'][t].data_ptr(),
                                logp=b['logp'][t].data_ptr(), action=b['action'][t].data_ptr(),
-                               workspace=_lib.ptr(ws), err=b['err'].data_ptr(), defer_heads=int(fuse_heads), **src)
+                               workspace=_lib.ptr(ws), err=b['err'].data_ptr(), **src)
             _lib.check(lib.ic3_policy_step(C.byref(cfg), C.byref(w), C.byref(io), s))
-            if fuse_heads:
-                heads_kw.update(head_value=b['value'][t].data_ptr(), head_logp=b['logp'][t].data_ptr())
             r = _lib.RolloutIO(t=t, max_steps=args.max_steps, nheads=nh, hard_attn=hard,
                                comm_action_one=int(bool(args.comm_action_one)),
                                last=int(t == T - 1 and quota <= 0), batch_size=int(quota),
-                               halted=b['halted'].data_ptr(), rec_valid=b['valid'].data_ptr(), **snap, **heads_kw,
+                               halted=b['halted'].data_ptr(), rec_valid=b['valid'].data_ptr(), **snap,
                                action=b['action'][t].data_ptr(), t_ep=b['t_ep'].data_ptr(),
                                fresh=b['fresh'].data_ptr(), comm_next=b['comm'].data_ptr(),
                                alive_next=b['alive'].data_ptr(), rec_reward=b['reward'].data_ptr(),

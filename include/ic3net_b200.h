@@ -137,15 +137,6 @@ typedef struct {
   uint8_t* snap_tj_alive;  /* [T, B, N] */
   uint8_t* snap_tj_last_act; /* [T, B, N] */
   int32_t* snap_tj_route_id; /* [T, B, N] */
-  /* Fused policy heads (tcgen05 path, ic3_policy_io.defer_heads): when head_partial != NULL the env step kernel first
-   * finishes the heads of this step from the LSTM epilogue's partial logits -- value, log-softmax, inverse-CDF sampling
-   * on the action stream of (cfg.seed, cfg.env_id0 + env, tick) -- writing head_value / head_logp and the `action`
-   * tensor (which is then an OUTPUT of the step, not an input), and consumes head 0 itself.  One launch less per step. */
-  const float* head_partial; /* ic3_policy_partial_ptr(...) */
-  const float* head_b;       /* ic3_policy_packed.head_b */
-  float* head_value;         /* [B*N] */
-  float* head_logp;          /* [B*N, sum(na)] */
-  int32_t head_dim[IC3_MAX_HEADS];
 } ic3_rollout_io;
 
 /* reset(): predator_prey_env.py:146-168.  Draws N+1 distinct cells per env from
@@ -278,11 +269,9 @@ typedef struct {
   float* head_b;   /* [1+sum(na)] */
   /* tcgen05 path (H == 128 only; both NULL selects the fp32 SIMT kernel):
    * lstm_img: fp16 hi/lo split of 256 * [W_ih ; W_ih.C ; W_hh] (K = 384) as ready-made
-   *   shared-memory images, [2 column halves][12 K-chunks][hi,lo][core-matrix layout] = 786432 bytes,
-   *   followed by a second copy of the same values in the layout of the 2-SM (cta_group::2) kernel,
-   *   [2 column halves][12 K-chunks][2 CTA ranks][hi,lo][core-matrix layout];
+   *   shared-memory images, [2 column halves][12 K-chunks][hi,lo][core-matrix layout] = 786432 bytes;
    * bias_cat: [4H] b_ih + b_hh + W_ih.c_b, column 4*u+gate.
-   * comm_passes > 1 (LSTM cell only): `passes` such image pairs / bias vectors one after the other, pass i folded
+   * comm_passes > 1 (LSTM cell only): `passes` such images / bias vectors one after the other, pass i folded
    *   with C_modules[i] (comm.py:63-70). */
   void* lstm_img;
   float* bias_cat;
@@ -294,7 +283,7 @@ typedef struct {
                       operand split), OR-ed into ic3_policy_io.err by every policy step; may be NULL */
 } ic3_policy_packed;
 
-#define IC3_LSTM_IMG_BYTES 1572864
+#define IC3_LSTM_IMG_BYTES 786432
 
 int ic3_policy_pack(const ic3_policy_cfg* cfg, const ic3_policy_params* p,
                     const ic3_policy_packed* out, void* stream);
@@ -342,16 +331,10 @@ typedef struct {
   /* optional, fused index encoder only: [positions, H] table of ic3_pp_encoder_table / ic3_tj_encoder_table
    * for the CURRENT weights (device pointer); needs cfg->obs_vocab > 0. */
   const float* x_table;
-  /* tcgen05 path with at most 7 action logits: 1 = stop after the LSTM kernel and leave the heads' partial logits in
-   * the workspace (ic3_policy_partial_ptr); the env step kernel finishes them (ic3_rollout_io.head_partial). */
-  int32_t defer_heads;
   int32_t pass_index;         /* callers pass 0.  comm_passes > 1 on the tcgen05 path: the library runs the step once per
                                  pass on a private copy of this struct and numbers the copies here (a fresh episode's
                                  zero state applies to pass 0 only; its masks to every pass, comm.py:179-218) */
 } ic3_policy_io;
-
-/* Partial-logit block inside a tcgen05 workspace (NULL when the configuration does not use it). */
-const float* ic3_policy_partial_ptr(const ic3_policy_cfg* cfg, const void* workspace);
 
 /* Scratch the tcgen05 policy path needs for a batch of cfg->B environments (0 when unsupported). */
 uint64_t ic3_policy_workspace_bytes(const ic3_policy_cfg* cfg);

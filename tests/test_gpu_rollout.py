@@ -236,21 +236,6 @@ def test_full_size_rollout_sampled_slots_match_oracle(name, B):
     replay_slots(args, z, p, batch, slots, T, seed, id0)
 
 
-@pytest.mark.parametrize("name", ["ep_pp_easy_ic3net", "ep_tj_medium_ic3net"])
-def test_heads_finished_by_the_env_step_kernel_equal_the_separate_kernel(name):
-    """args.fuse_heads: the env step kernel finishes value / log-probs / sampling from the LSTM epilogue's partial
-    logits (ic3_rollout_io.head_partial).  Same arithmetic in the same order -> bit-identical records."""
-    meta, z = load_golden(name)
-    res = []
-    for fuse in (False, True):
-        args, env, net, tr, p = build(meta, 20, "index", seed=31, fuse_heads=fuse)
-        b = tr.rollout(30, 0)
-        tr.collect_stat()
-        res.append((cpu(b.action).copy(), cpu(b.value).copy(), cpu(b.logp).copy(), cpu(b.reward).copy()))
-    for x, y in zip(res[0], res[1]):
-        assert np.array_equal(x, y)
-
-
 @pytest.mark.parametrize("name,impl", [("ep_pp_hard_ic3net", "tc"), ("ep_tj_medium_ic3net", "tc"), ("ep_pp_easy_ic3net", "simt"),
                                        ("ep_tj_medium_v1_commnet", "simt")])
 def test_observation_handle_api_is_bit_identical_to_the_dense_tensor_api(name, impl):
